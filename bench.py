@@ -3,6 +3,8 @@
 + dB) in window-features/s -- BASELINE.json's metric -- on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                       also write the last timed step's outputs
+                                                               (seeded inputs: comparable across builds)
   python bench.py --impl reference ...                         the reference's CPU path
                                                                (oracle port: the reference
                                                                itself cannot be imported here)
@@ -307,6 +309,24 @@ def measure_note_step(torch, ops, synth, dev, n_windows=600, steps=5):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+DUMP_WINDOWS = 8        # mag + D of 8 windows: 34 MB of float32
+
+
+def dump_outputs(torch, pipe, out_dir, seed=0):
+    """Write what the last step returned to its caller as float32 `out_dir/<name>.npy`: `ref` [W], the
+    post-subtraction ref_mag of every window, and for a fixed seeded sample of DUMP_WINDOWS windows (ascending
+    window order) `mag` [n, frames, bins], the subtracted STFT magnitude, `D` [n, frames, bins], its dB image, and
+    `C` [n, frames, cqt bins], the constant-Q magnitudes.  The inputs are seeded as well, so two builds run with
+    the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(seed).choice(pipe.W, size=min(DUMP_WINDOWS, pipe.W), replace=False))
+    sel = torch.as_tensor(idx, device=pipe.dev)
+    out = {"ref": pipe.ref, "mag": pipe.mag[sel, :pipe.T, :pipe.nb], "D": pipe.D[sel, :pipe.T, :pipe.nb],
+           "C": pipe.C[sel, :, :pipe.cqt.n_bins]}
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(torch.float32).cpu().numpy())
+
+
 def bind_to_gpu_cpus(local):
     """Pin this rank to the CPUs NVML reports as local to its GPU, so that the pinned host buffers of the end-to-end
     path are allocated (first touch) on the GPU's own NUMA node and the H2D copies of eight ranks do not all cross
@@ -396,6 +416,8 @@ def run_saga(args):
     barrier()
     launches = ops.launch_count() - launches0
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:     # before the passes below overwrite the pipeline's buffers
+        dump_outputs(torch, pipe, args.dump_outputs)
     # per-kernel durations for the roofline: the same steps again with the two chains of the path run one
     # after the other (in the timed loop above the CQT chain overlaps the STFT / subtract chain on a second
     # stream, so a kernel's own duration cannot be read off there)
@@ -699,6 +721,9 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=12, help="window chunks for H2D/compute/D2H overlap")
     ap.add_argument("--no-ref-shape", action="store_true", help="skip the extra pass at the reference's default n_fft/hop")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg4 chain and batched per-note measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32; "
+                         "ref_mag of every window, mag / D / C of a fixed sample of %d windows)" % DUMP_WINDOWS)
     ap.add_argument("--cfg5-hours", type=float, default=0.0,
                     help="BASELINE config 5 instead of the step bench: this many hours of synthetic audio (360 clips of 10 s per "
                          "hour), block-partitioned over the ranks, generated on device in 1 h chunks, STFT + CQT, checksum gathered")

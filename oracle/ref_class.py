@@ -36,12 +36,13 @@ import numpy as _np
 from . import cqt as _cqt
 from . import spectral as _sp
 
-REFERENCE_DIR = os.environ.get("SAGA_REFERENCE_DIR", "/root/reference")
+# a checkout of the original project (its util_audio.py and fixture directories); unset: not available
+REFERENCE_DIR = os.environ.get("SAGA_REFERENCE_DIR", "")
 _mod = None
 
 
 def available():
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "util_audio.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "util_audio.py"))
 
 
 class _NumpyWithInt:
@@ -88,12 +89,12 @@ def _stubs():
 
 
 def load():
-    """Import /root/reference/util_audio.py (once) and return the module."""
+    """Import the original project's util_audio.py (once) and return the module."""
     global _mod
     if _mod is not None:
         return _mod
     if not available():
-        raise FileNotFoundError("reference not present at %s (expected on the GPU box)" % REFERENCE_DIR)
+        raise FileNotFoundError("SAGA_REFERENCE_DIR does not name the original project's source (%r)" % REFERENCE_DIR)
     stand_ins = _stubs()
     saved = {n: sys.modules.get(n) for n in stand_ins}
     sys.modules.update(stand_ins)

@@ -40,8 +40,10 @@ def test_batched_note_step_matches_reference_class_golden(full_cqt):
     import amt_saga_b200  # noqa: F401
     from amt_saga_b200 import util_audio as ua
     from amt_saga_b200.note_step import NoteStepBatch
-    gold = dict(np.load(os.path.join(GOLD, "ref_class_note_steps.npz")))
     W = len(NOTE_STEPS)
+    gold = {}
+    for w in range(W):
+        gold.update(np.load(os.path.join(GOLD, "ref_class_note_steps_w%d.npz" % w)))
     songs, clips = zip(*[L.make_inputs(c["seed"], c["seconds"], c["notes"]) for c in NOTE_STEPS])
     # windows exactly as `mid_wf.section(0, None, 258)` leaves them (training.py:284)
     mags, phs, wavs = [], [], []

@@ -20,10 +20,11 @@ import pytest
 from oracle import ref_class
 from oracle.audio_oracle import AudioOracle
 from tests import ref_loop as L
-from tests.golden.make_ref_class_golden import FULL, FULL_COLS, SMALL, thin
+from tests.golden.make_ref_class_golden import FULL, FULL_COLS, SMALL, thin, thin_small
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-needs_reference = pytest.mark.skipif(not ref_class.available(), reason="/root/reference not mounted (GPU box)")
+needs_reference = pytest.mark.skipif(not ref_class.available(),
+                                     reason="needs the original project's source: set SAGA_REFERENCE_DIR")
 MAG_TOL, DB_TOL = 1e-4, 0.01
 
 
@@ -44,7 +45,7 @@ def _assert_identical(a, b):
 @needs_reference
 def test_reference_class_imports_unmodified():
     m = ref_class.load()
-    assert os.path.samefile(m.__file__, "/root/reference/util_audio.py")
+    assert os.path.samefile(m.__file__, os.path.join(ref_class.REFERENCE_DIR, "util_audio.py"))
     ac = m.audio_complete(np.zeros(8192), 4096)
     assert ac.hl == 1024 and ac.shape == (2049, 9)          # util_audio.py:65, T = 1 + n // hop
 
@@ -91,7 +92,7 @@ def test_static_helpers_equal_reference_class():
 
 def test_oracle_matches_committed_reference_class_golden_small():
     g = dict(np.load(os.path.join(GOLD, "ref_class_loop_small.npz")))
-    _assert_identical(g, _run(AudioOracle, SMALL))
+    _assert_identical(g, thin_small(_run(AudioOracle, SMALL)))
 
 
 def test_oracle_matches_committed_reference_class_golden_setters():
@@ -122,6 +123,8 @@ def _compare_with_golden(got, gold):
         v = got[k]
         assert v.shape == g.shape, k
         base = k.split("_", 1)[1] if k[0] == "n" and k[1].isdigit() else k
+        if base.endswith("__sha256"):   # bit patterns: checked on the CPU container only
+            continue
         if base in EXACT:
             assert np.array_equal(v, g), k
         elif base == "D_final" or base.startswith("D_final__c"):
@@ -155,7 +158,7 @@ def _compare_with_golden(got, gold):
 @pytest.mark.gpu
 def test_cuda_class_matches_reference_class_golden_small(cuda_class):
     gold = dict(np.load(os.path.join(GOLD, "ref_class_loop_small.npz")))
-    _compare_with_golden(_run(cuda_class, SMALL), gold)
+    _compare_with_golden(thin_small(_run(cuda_class, SMALL)), gold)
 
 
 @pytest.mark.gpu

@@ -1,12 +1,13 @@
 """Pins against the reference's OWN outputs.
 
 `subtraction_demo/<name>_test{,_guess,_sub}.flac` are waveforms the reference wrote itself
-(`/root/reference/test_snippets.py:473-514`, saved through `util_audio.py:520-527`): the mix, the
+(`test_snippets.py:473-514`, saved through `util_audio.py:520-527`): the mix, the
 guessed note, and `istft(relu(mag - shifted normalised guess) * ph)`.  Decoded with the test-only
 FLAC reader they pin  STFT -> magphase -> ref_mag -> subtract -> iSTFT  end to end: the oracle (and,
 on a GPU, the CUDA path through the C ABI) must reproduce `_sub` from `_test` and `_guess` to the
 24-bit quantisation of the files.  One triple is committed as tests/golden/ref_subtraction_piano.npz
-(tests/golden/make_reference_pins.py); the others are checked when /root/reference is mounted.
+(tests/golden/make_reference_pins.py); the others are checked when SAGA_REFERENCE_DIR names a
+checkout of the original project.
 """
 import json
 import os
@@ -14,11 +15,12 @@ import os
 import numpy as np
 import pytest
 
+from oracle import ref_class
 from oracle.audio_oracle import AudioOracle
 from tests.flac_reader import read_flac
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-DEMO = "/root/reference/subtraction_demo/"
+DEMO = os.path.join(ref_class.REFERENCE_DIR, "subtraction_demo", "")
 SCALE = float(1 << 23)
 # both inputs and the output went through 24-bit rounding: the residual is a few LSB at most and about
 # a third of an LSB rms (measured: tests/golden/ref_subtraction_pins.json)
@@ -59,7 +61,11 @@ def test_wrong_parameters_do_not_reproduce_it():
     assert mx > 1e4
 
 
-@pytest.mark.skipif(not os.path.isdir(DEMO), reason="reference fixtures are only mounted in the build container")
+needs_fixtures = pytest.mark.skipif(not (ref_class.REFERENCE_DIR and os.path.isdir(DEMO)),
+                                    reason="needs the original project's FLAC fixtures: set SAGA_REFERENCE_DIR")
+
+
+@needs_fixtures
 @pytest.mark.parametrize("name", sorted(PINS))
 def test_oracle_reproduces_reference_subtraction_from_flac(name):
     pcm = {}
@@ -73,11 +79,11 @@ def test_oracle_reproduces_reference_subtraction_from_flac(name):
     assert mx <= MAX_LSB and rms <= RMS_LSB, (mx, rms)
 
 
-@pytest.mark.skipif(not os.path.isdir(DEMO), reason="reference fixtures are only mounted in the build container")
+@needs_fixtures
 def test_fixture_lengths_pin_resize_targets():
     """short_window_demo/{j}/sw_{j}_*.flac hold exactly 1024*(j-1) samples: `_resize` returned j frames
     (test_snippets.py:1204-1211) and istft yields hop*(T-1) samples."""
-    root = "/root/reference/short_window_demo/"
+    root = os.path.join(ref_class.REFERENCE_DIR, "short_window_demo", "")
     for j in (6, 8, 10, 15, 20):
         pcm, sr, bps = read_flac(root + "%d/sw_%d_0.flac" % (j, j))
         assert len(pcm) == 1024 * (j - 1) and sr == 44100
