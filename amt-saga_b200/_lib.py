@@ -59,6 +59,8 @@ SIGNATURES = {
     "saga_cqt_frames_exec": (_I, [_P, _P, _P, _P, _I, _L, _P, _I, _P, _L, _L, _P, _L, _P]),
     "saga_cqt_frames_shared_exec": (_I, [_P, _P, _P, _P, _I, _L, _I, _I, _I, _P, _I, _P, _L, _L, _P, _L, _P]),
     "saga_cqt_frames_shared_multi_exec": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _L, _P, _I, _P, _L, _L, _P, _L, _P]),
+    "saga_cqt_peak_workspace_bytes": (_L, [_P, _I, _L]),
+    "saga_cqt_peak_exec": (_I, [_P, _P, _P, _P, _I, _L, _P, _P, _P, _P, _L, _P]),
     "saga_compress_bands_exec": (_I, [_P, _P, _P, _I, _I, _I, _L, _L, _L, _L, _P, _P]),
     "saga_short_window_exec": (_I, [_P, _P, _P, _I, _I, _I, _I, _L, _F, _P, _P, _P, _L, _P]),
     "saga_short_window_batch_exec": (_I, [_P, _P, _L, _L, _P, _I, _P, _I, _I, _I, _P, _F, _P, _P, _P, _L, _L, _I, _P]),

@@ -72,5 +72,6 @@ extern "C" const char* saga_get_option(const char* name) { return name ? saga::o
 extern "C" const char* saga_last_error_string(void) { return saga::err_buf(); }
 // 2: + saga_short_window_batch_exec, saga_gather_frames_exec, saga_cqt_frames_exec, saga_set/get_option
 // 3: + saga_cqt_frames_shared_exec, saga_cqt_frames_shared_multi_exec, saga_istft_rows_exec (additions only)
+//    + saga_cqt_peak_workspace_bytes, saga_cqt_peak_exec (additions only: existing entries unchanged)
 extern "C" int saga_abi_version(void) { return 3; }
 extern "C" int64_t saga_launch_count(void) { return saga::g_launches.load(); }

@@ -1334,3 +1334,111 @@ extern "C" int saga_cqt_frames_exec(const saga_cqt_plan* p, const float* wav, co
   return cqt_exec_impl(p, wav, clip_offsets, clip_lens, n_clips, max_len, C_mag_out, nullptr, frame_pitch,
                        out_clip_stride, workspace, workspace_bytes, 1, stream, frame_first, frame_count);
 }
+
+// ---------------------------------------------------------------------------
+// Peak of a column range per clip (saga_cqt_peak_exec): the whole-song normalisers of the producer loop
+// (training.py:271-282) are np.max of `C[:, 0:t]` of a full transform.  Plans the streamed tensor-core kernel runs
+// contract in its peak mode (packed rows, no image); every other plan contracts into an image in the workspace that
+// cqt_column_peak_kernel reduces.
+// ---------------------------------------------------------------------------
+namespace saga {
+
+// row_start[c] = sum of the frame counts of clips < c, row_start[n_clips] = all rows (one thread: a batch is songs)
+__global__ void cqt_row_start_kernel(const int32_t* clip_frames, int n_clips, int32_t* row_start) {
+  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+  int32_t s = 0;
+  for (int c = 0; c < n_clips; ++c) {
+    row_start[c] = s;
+    s += clip_frames[c];
+  }
+  row_start[n_clips] = s;
+}
+
+// max over bins [0, n_bins) and frames [max(col_lo, 0), min(col_hi, T_c)) of clip blockIdx.y of a frame-major image
+__global__ void __launch_bounds__(256) cqt_column_peak_kernel(const float* img, int64_t frame_pitch, int64_t clip_stride,
+                                                             int n_bins, const int32_t* clip_frames, const int32_t* col_lo,
+                                                             const int32_t* col_hi, unsigned int* peak_out) {
+  const int c = blockIdx.y;
+  const int lo = max(col_lo[c], 0), hi = min(col_hi[c], clip_frames[c]);
+  float m = 0.f;
+  for (int t = lo + blockIdx.x * blockDim.y + threadIdx.y; t < hi; t += gridDim.x * blockDim.y)
+    for (int k = threadIdx.x; k < n_bins; k += blockDim.x) m = fmaxf(m, img[c * clip_stride + t * frame_pitch + k]);
+  m = warp_max(m);
+  if (threadIdx.x == 0 && m > 0.f) atomicMax(peak_out + c, __float_as_uint(m));      // magnitudes >= 0: bit order
+}
+
+static int64_t round256(int64_t b) { return (b + 255) & ~int64_t(255); }
+
+// the plans saga_cqt_exec contracts with the streamed kernel (the resident kernel declines them and the option allows it)
+static bool peak_streamed(const saga_cqt_plan* p) {
+  const char* opt = SAGA_OPT("SAGA_CQT_STREAM");
+  return cqt_stream_supported(p) && !cqt_umma_supported(p) && !(opt && atoi(opt) == 0);
+}
+
+}  // namespace saga
+
+extern "C" int64_t saga_cqt_peak_workspace_bytes(const saga_cqt_plan* p, int n_clips, int64_t max_len) {
+  if (!p || n_clips <= 0 || max_len <= 0) return 256;
+  int64_t b = round256(saga_cqt_workspace_bytes(p, n_clips, max_len)) + round256(((int64_t)n_clips + 1) * 4);
+  if (!peak_streamed(p)) b += (int64_t)n_clips * saga_cqt_num_frames(p, max_len) * ((p->n_bins + 3) & ~3) * 4;
+  return b;
+}
+
+extern "C" int saga_cqt_peak_exec(const saga_cqt_plan* p, const float* wav, const int64_t* clip_offsets,
+                                  const int64_t* clip_lens, int n_clips, int64_t max_len, const int32_t* col_lo,
+                                  const int32_t* col_hi, float* peak_out, void* workspace, int64_t workspace_bytes,
+                                  void* stream) {
+  if (!p || !wav || !clip_offsets || !col_lo || !col_hi || !peak_out || !workspace)
+    return set_error(SAGA_ERR_INVALID, "cqt_peak_exec: null argument");
+  if (n_clips < 0) return set_error(SAGA_ERR_INVALID, "cqt_peak_exec: n_clips < 0");
+  if (n_clips == 0) return SAGA_OK;
+  if (workspace_bytes < saga_cqt_peak_workspace_bytes(p, n_clips, max_len))
+    return set_error(SAGA_ERR_INVALID, "cqt_peak_exec: workspace too small");
+  if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0)
+    return set_error(SAGA_ERR_INVALID, "cqt_peak_exec: workspace must be 256-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  SAGA_CUDA_OK(cudaMemsetAsync(peak_out, 0, sizeof(float) * n_clips, st));
+  if (max_len <= 0) return SAGA_OK;
+  const int64_t T_max = saga_cqt_num_frames(p, max_len);
+  char* ws = (char*)workspace;
+  const int64_t cqt_bytes = round256(saga_cqt_workspace_bytes(p, n_clips, max_len));
+  int32_t* row_start = (int32_t*)(ws + cqt_bytes);
+  const int32_t* clip_frames = (const int32_t*)ws;          // header of the cascade's workspace (cqt_exec_impl)
+  unsigned int* peak_bits = reinterpret_cast<unsigned int*>(peak_out);
+  if (!peak_streamed(p)) {
+    float* img = (float*)(ws + cqt_bytes + round256(((int64_t)n_clips + 1) * 4));
+    const int64_t P = (p->n_bins + 3) & ~3;
+    const int rc = cqt_exec_impl(p, wav, clip_offsets, clip_lens, n_clips, max_len, img, nullptr, P, T_max * P, workspace,
+                                 cqt_bytes, 0, stream, nullptr, 0);
+    if (rc != SAGA_OK) return rc;
+    dim3 grid((unsigned)std::min<int64_t>((T_max + 7) / 8, 64), n_clips), block(32, 8);
+    cqt_column_peak_kernel<<<grid, block, 0, st>>>(img, P, T_max * P, p->n_bins, clip_frames, col_lo, col_hi, peak_bits);
+    SAGA_LAUNCH_CHECK();
+    return SAGA_OK;
+  }
+  // cascade + reflect margins exactly as saga_cqt_exec runs them, then the contraction in peak mode
+  static float dummy;
+  int rc = cqt_exec_impl(p, wav, clip_offsets, clip_lens, n_clips, max_len, &dummy, nullptr, p->n_bins, 0, workspace,
+                         cqt_bytes, SAGA_CQT_SKIP_CONTRACT, stream, nullptr, 0);
+  if (rc != SAGA_OK) return rc;
+  if (p->max_level + 1 > PAD_MAX_LEVELS) return set_error(SAGA_ERR_UNSUPPORTED, "cqt_peak_exec: too many levels");
+  // the workspace layout of cqt_exec_impl
+  std::vector<float*> lvl(p->max_level + 1, nullptr);
+  std::vector<int64_t> pitch(p->max_level + 1, 0);
+  std::vector<int> pad(p->max_level + 1, 0);
+  char* w = ws + ws_header_bytes(n_clips);
+  for (int l = 0; l <= p->max_level; ++l) {
+    pitch[l] = cqt_level_pitch(p, l, max_len);
+    pad[l] = cqt_level_pad(p, l);
+    lvl[l] = (float*)w;
+    w += (int64_t)n_clips * pitch[l] * 4;
+  }
+  CqtLevels lv;
+  lv.wav = wav; lv.clip_offsets = clip_offsets; lv.clip_lens = clip_lens; lv.max_len = max_len;
+  lv.lvl = lvl.data(); lv.pitch = pitch.data(); lv.pad = pad.data(); lv.clip_frames = clip_frames;
+  cqt_row_start_kernel<<<1, 32, 0, st>>>(clip_frames, n_clips, row_start);
+  SAGA_LAUNCH_CHECK();
+  CqtPeakArgs pk;
+  pk.row_start = row_start; pk.col_lo = col_lo; pk.col_hi = col_hi; pk.peak_out = peak_out;
+  return cqt_stream_peak_exec(p, lv, n_clips, T_max, pk, st);
+}

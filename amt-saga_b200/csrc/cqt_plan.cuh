@@ -65,11 +65,21 @@ int cqt_stream_exec(const saga_cqt_plan* p, const CqtLevels& lv, int n_clips, in
                     const int32_t* frame_first, int frame_count, float* mag_out, float2* cplx_out,
                     int64_t frame_pitch, int64_t out_clip_stride, cudaStream_t st, int max_slices = 1,
                     float* partial = nullptr, int pstride = 0, int* slices_out = nullptr);
+// peak mode of the streamed kernel (saga_cqt_peak_exec): rows packed through the device prefix sum row_start[n_clips + 1]
+// of the clip frame counts, peak_out[c] = max |C| over bins and frames col_lo[c] <= t < col_hi[c] (peak_out zeroed before)
+struct CqtPeakArgs {
+  const int32_t* row_start;
+  const int32_t* col_lo;
+  const int32_t* col_hi;
+  float* peak_out;
+};
 // several plans of equal geometry, plan i on clips [clip0[i], clip0[i] + nclips[i]) of the batch `lv` describes
 int cqt_stream_exec_multi(const saga_cqt_plan* const* plans, int n_plans, const int* clip0, const int* nclips,
                           const CqtLevels& lv, int n_clips, int64_t T_max, const int32_t* frame_first, int frame_count,
                           float* mag_out, float2* cplx_out, int64_t frame_pitch, int64_t out_clip_stride,
                           cudaStream_t st, int max_slices = 1, float* partial = nullptr, int pstride = 0,
-                          int* slices_out = nullptr);
+                          int* slices_out = nullptr, const CqtPeakArgs* peak = nullptr);
+int cqt_stream_peak_exec(const saga_cqt_plan* p, const CqtLevels& lv, int n_clips, int64_t T_max, const CqtPeakArgs& peak,
+                         cudaStream_t st);
 
 }  // namespace saga

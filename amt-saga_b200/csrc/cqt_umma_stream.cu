@@ -21,7 +21,10 @@
 //   * whole transforms  : rows = every frame of every clip, 128 consecutive (clip, frame) pairs per tile --
 //                         clips of 258 frames pack densely, there are no partial tiles and no tail kernel;
 //   * frame windows     : rows = frames [first[clip], first[clip] + 8) of every clip (saga_cqt_frames_exec: the
-//                         producer loop keeps 8 columns of each per-note transform), 16 clips per tile.
+//                         producer loop keeps 8 columns of each per-note transform), 16 clips per tile;
+//   * column-range peaks: rows = the frames of every clip PACKED back to back (a device prefix sum of the clip frame
+//                         counts, so ragged clips cost their own frames, not T_max each), nothing stored: the
+//                         epilogue keeps max |C| per clip (saga_cqt_peak_exec, the kernel's PEAK instantiation).
 // Column groups of <= 128 real columns (64 filters) are separate work items, ordered (octave, group)-major so
 // that all CTAs stream the same bank slab out of L2 at the same time.  A work item's group also names its clip
 // range and bank, so one launch can contract several plans of equal geometry (one bank per pitch:
@@ -105,6 +108,15 @@ struct UsArgs {
   // [slice][clip][octave][pstride filters][8 frames][re, im] for cqt_frame_window_finish_kernel (cqt.cu)
   int ks, n_oct, pstride;
   float* partial;
+  // peak mode (saga_cqt_peak_exec): PACKED rows -- row R is frame R - row_start[c] of the clip c with
+  // row_start[c] <= R < row_start[c + 1] (device prefix sum of the clip frame counts, row_start[n_clips] = all rows), so
+  // every group has ceil(row_start[n_clips] / 128) tiles, read by every role at kernel start.  Nothing is stored: the
+  // epilogue folds max |C| over the bins of each row with col_lo[c] <= t < col_hi[c] into peak_out[c] (atomicMax on the
+  // bits of a float >= 0; peak_out zeroed by the caller)
+  const int32_t* row_start;     // NULL = not peak mode
+  const int32_t* col_lo;
+  const int32_t* col_hi;
+  unsigned int* peak_out;
   int debug;                    // SAGA_UMMA_DEBUG (timing bisection only): 1 no MMAs, 2 no row copies, 8 no bank copies, 32 no lo conversion
   int* error_flag;
   long long* prof;              // debug & 16: per-CTA cycle counters [grid][8]
@@ -119,8 +131,16 @@ struct UsRow {
 struct UsItem {
   uint32_t g, slice, tile;
 };
-__device__ __forceinline__ UsItem us_item(const UsArgs& a, uint32_t item) {
+// peak mode: `ptiles` = packed tiles per group (every group covers all rows once, ks = 1)
+template <bool PEAK>
+__device__ __forceinline__ UsItem us_item(const UsArgs& a, uint32_t item, uint32_t ptiles) {
   UsItem it;
+  if (PEAK) {
+    it.g = item / ptiles;
+    it.slice = 0;
+    it.tile = item - it.g * ptiles;
+    return it;
+  }
   uint32_t g = 0;
   while (g + 1 < (uint32_t)a.n_groups && item >= a.grp[g + 1].item0) ++g;
   const uint32_t local = item - a.grp[g].item0, tiles = a.grp[g].tiles;
@@ -129,8 +149,26 @@ __device__ __forceinline__ UsItem us_item(const UsArgs& a, uint32_t item) {
   it.tile = local - it.slice * tiles;
   return it;
 }
+template <bool PEAK>
 __device__ __forceinline__ UsRow us_row(const UsArgs& a, const UsGroup& gr, uint32_t R) {
   UsRow r;
+  if (PEAK) {
+    // packed rows: the last clip whose first row is <= R (clips without frames share their successor's row_start)
+    const uint32_t n_rows = (uint32_t)a.row_start[a.n_clips];
+    if (R >= n_rows) {
+      r.clip = 0; r.j = 0; r.t = 0; r.store = false; r.live = false;
+      return r;
+    }
+    int lo = 0, hi = a.n_clips - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if ((uint32_t)a.row_start[mid] <= R) lo = mid; else hi = mid - 1;
+    }
+    r.clip = lo;
+    r.j = r.t = (int)(R - (uint32_t)a.row_start[lo]);
+    r.store = r.live = true;
+    return r;
+  }
   if (R >= gr.n_rows) {
     r.clip = gr.clip0; r.j = 0; r.t = 0; r.store = false; r.live = false;
     return r;
@@ -300,6 +338,7 @@ __device__ __forceinline__ void us_wait(uint64_t* bar, uint32_t parity, int lane
   while (!us_test_wait(bar, parity)) {}
 }
 
+template <bool PEAK>
 __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __grid_constant__ UsArgs a) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t S = (uint32_t)a.stages;
@@ -337,23 +376,29 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_ptr_s, 0);
   const uint32_t G = gridDim.x;
+  // peak mode: the packed row count is known on the device only (every role reads the same value)
+  const uint32_t ptiles = PEAK ? ((uint32_t)a.row_start[a.n_clips] + US_TILE_M - 1) / US_TILE_M : 0u;
+#define US_TOTAL_ITEMS (PEAK ? (uint32_t)a.n_groups * ptiles : a.total_items)
 
   if (warp < 4) {
     // =========================== epilogue ===========================
     const int ew = warp;
     uint32_t it_acc = 0;
-    for (uint32_t item = blockIdx.x; item < a.total_items; item += G, ++it_acc) {
-      const UsItem wi = us_item(a, item);
+    for (uint32_t item = blockIdx.x; item < US_TOTAL_ITEMS; item += G, ++it_acc) {
+      const UsItem wi = us_item<PEAK>(a, item, ptiles);
       const uint32_t g = wi.g, slice = wi.slice, tile = wi.tile;
       const UsGroup& gr = a.grp[g];
       const uint32_t acc = a.bufs == 2 ? (it_acc & 1) : 0, acc_ph = a.bufs == 2 ? ((it_acc >> 1) & 1) : (it_acc & 1);
-      const UsRow r = us_row(a, gr, tile * US_TILE_M + (uint32_t)(ew * 32 + lane));
+      const UsRow r = us_row<PEAK>(a, gr, tile * US_TILE_M + (uint32_t)(ew * 32 + lane));
       us_wait(&tfull[acc], acc_ph, lane, a.error_flag, 500);
       tc_fence_after();
       const int64_t row = (int64_t)r.clip * a.out_clip_stride + (int64_t)(a.frame_first ? r.j : r.t) * a.frame_pitch;
       const uint32_t tbase = tmem_base + acc * a.acc_stride + ((uint32_t)(ew * 32) << 16);
       const bool vec_ok = ((a.frame_pitch | a.out_clip_stride | (int64_t)gr.first_bin) & 3) == 0 && !a.cplx_out &&
                           (reinterpret_cast<uintptr_t>(a.mag_out) & 15) == 0;
+      // peak mode: the row counts when its frame lies in the clip's column range
+      const bool in_range = PEAK && r.live && r.t >= a.col_lo[r.clip] && r.t < a.col_hi[r.clip];
+      float peak = 0.f;
       for (int c0 = 0; c0 < gr.ncol; c0 += 8) {
         float hi[8], lo[8];
 #pragma unroll
@@ -369,7 +414,20 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
             lo[i] += __uint_as_float(u[i]);
           }
         }
-        if (a.ks > 1) {
+        if (PEAK) {
+          // the storing path's arithmetic below, folded into a maximum instead of stored
+          if (in_range) {
+            float sum[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) sum[i] = hi[i] + lo[i];
+            const int bin0 = gr.first_bin + (c0 >> 1);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              const int bin = bin0 + i;
+              if (bin >= 0 && bin < a.n_bins) peak = fmaxf(peak, sqrtf(sum[2 * i] * sum[2 * i] + sum[2 * i + 1] * sum[2 * i + 1]));
+            }
+          }
+        } else if (a.ks > 1) {
           if (r.store) {
             float2* dst = reinterpret_cast<float2*>(
                 a.partial + ((((int64_t)slice * a.n_clips + r.clip) * a.n_oct + gr.oct) * a.pstride + gr.filt0 + (c0 >> 1)) * 16) + r.j;
@@ -401,6 +459,13 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty[acc]);
+      if (PEAK) {
+        // the lanes of one clip (a warp's 32 consecutive rows span one or a few clips) reduce first: one atomic per
+        // clip and warp.  Magnitudes are >= 0, so the order of their bit patterns as integers is the float order.
+        const unsigned same = __match_any_sync(0xffffffffu, in_range ? r.clip : -1);
+        const unsigned bits = __reduce_max_sync(same, in_range ? __float_as_uint(peak) : 0u);
+        if (in_range && lane == __ffs(same) - 1 && bits != 0u) atomicMax(a.peak_out + r.clip, bits);
+      }
     }
   } else if (warp == US_W_MMA || warp == US_W_MMA2) {
     // =========================== MMA issuer(s) ===========================
@@ -417,8 +482,8 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
     const long long pt_start = pt;
 #define US_PROF(var) do { if (prof_on) { const long long n_ = clock64(); var += n_ - pt; pt = n_; } } while (0)
 #define US_TL(kk, slot) do { if ((a.debug & 128) && blockIdx.x == 0 && lane == 0 && (kk) < 96u) a.prof[2048 + (kk) * 8 + (slot)] = clock64(); } while (0)
-    for (uint32_t item = blockIdx.x; item < a.total_items; item += G, ++it_acc) {
-      const uint32_t g = us_item(a, item).g;
+    for (uint32_t item = blockIdx.x; item < US_TOTAL_ITEMS; item += G, ++it_acc) {
+      const uint32_t g = us_item<PEAK>(a, item, ptiles).g;
       const UsGroup& gr = a.grp[g];
       // (k runs over THIS issuer's stages: iw, iw + NI, ... across items; every item has a multiple of 4 stages)
       // instruction descriptors: D = f32, A = B = tf32, K-major both, M = 128
@@ -514,8 +579,8 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
     // =========================== bank loader ===========================
     if (lane == 0) {
       uint32_t k = 0;
-      for (uint32_t item = blockIdx.x; item < a.total_items; item += G) {
-        const UsItem wi = us_item(a, item);
+      for (uint32_t item = blockIdx.x; item < US_TOTAL_ITEMS; item += G) {
+        const UsItem wi = us_item<PEAK>(a, item, ptiles);
         const uint32_t g = wi.g, slice = wi.slice;
         const UsGroup& gr = a.grp[g];
         const uint32_t bytes = (uint32_t)gr.n_main * (US_PLANES * 16u);
@@ -552,12 +617,12 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
       const int k_off = sub * nk;
       const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
       uint32_t k0t = 0;
-      for (uint32_t item = blockIdx.x; item < a.total_items; item += G) {
-        const UsItem wi = us_item(a, item);
+      for (uint32_t item = blockIdx.x; item < US_TOTAL_ITEMS; item += G) {
+        const UsItem wi = us_item<PEAK>(a, item, ptiles);
         const uint32_t g = wi.g, slice = wi.slice, tile = wi.tile;
         const UsGroup& gr = a.grp[g];
         const int n_st = gr.n_fft / US_KC / a.ks;
-        const UsRow r = us_row(a, gr, tile * US_TILE_M + (uint32_t)row);
+        const UsRow r = us_row<PEAK>(a, gr, tile * US_TILE_M + (uint32_t)row);
         const int T = a.clip_frames[r.clip];
         const int tc = max(min(r.t, T - 1), 0);      // frames outside the clip re-read an existing one (never stored)
         const float* own = gr.sig + (int64_t)r.clip * gr.sig_stride + (int64_t)tc * gr.hop + (int)slice * n_st * US_KC + k_off;
@@ -614,15 +679,15 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
     const int plane = t & 7, row0 = t >> 3;
     const uint32_t dst_off = (uint32_t)plane * US_PLANE_BYTES + (uint32_t)row0 * 16u;
     uint32_t k0 = 0;                                   // ring index of the item's first stage
-    for (uint32_t item = blockIdx.x; item < a.total_items; item += G) {
-      const UsItem wi = us_item(a, item);
+    for (uint32_t item = blockIdx.x; item < US_TOTAL_ITEMS; item += G) {
+      const UsItem wi = us_item<PEAK>(a, item, ptiles);
       const uint32_t g = wi.g, slice = wi.slice, tile = wi.tile;
       const UsGroup& gr = a.grp[g];
       const int n_st = gr.n_fft / US_KC / a.ks;
       const float4* src[US_MAX_RPT];
 #pragma unroll
       for (int i = 0; i < US_MAX_RPT; ++i) {
-        const UsRow r = us_row(a, gr, tile * US_TILE_M + (uint32_t)(row0 + rstep * (i < rpt ? i : 0)));
+        const UsRow r = us_row<PEAK>(a, gr, tile * US_TILE_M + (uint32_t)(row0 + rstep * (i < rpt ? i : 0)));
         const int T = a.clip_frames[r.clip];
         const int tc = max(min(r.t, T - 1), 0);      // frames outside the clip re-read an existing one (never stored)
         src[i] = reinterpret_cast<const float4*>(gr.sig + (int64_t)r.clip * gr.sig_stride + (int64_t)tc * gr.hop + 4 * plane +
@@ -672,6 +737,7 @@ __global__ void __launch_bounds__(US_THREADS, 1) cqt_umma_stream_kernel(const __
     }   // shared-memory A
   }
 
+#undef US_TOTAL_ITEMS
   tc_fence_before();
   __syncthreads();
   if (warp == 0) {
@@ -812,7 +878,8 @@ void cqt_stream_plan_init(saga_cqt_plan* p) {
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&st->num_sms, cudaDevAttrMultiProcessorCount, dev);
   // the attribute is per function, plans differ in their needs: ask for the maximum once
-  if (cudaFuncSetAttribute(cqt_umma_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)US_SMEM_LIMIT) != cudaSuccess) {
+  if (cudaFuncSetAttribute(cqt_umma_stream_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)US_SMEM_LIMIT) != cudaSuccess ||
+      cudaFuncSetAttribute(cqt_umma_stream_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)US_SMEM_LIMIT) != cudaSuccess) {
     cudaGetLastError();
     return;
   }
@@ -839,13 +906,21 @@ int cqt_stream_exec(const saga_cqt_plan* p, const CqtLevels& lv, int n_clips, in
                                frame_pitch, out_clip_stride, stream, max_slices, partial, pstride, slices_out);
 }
 
+int cqt_stream_peak_exec(const saga_cqt_plan* p, const CqtLevels& lv, int n_clips, int64_t T_max, const CqtPeakArgs& peak,
+                         cudaStream_t stream) {
+  const int zero = 0;
+  return cqt_stream_exec_multi(&p, 1, &zero, &n_clips, lv, n_clips, T_max, nullptr, 0, nullptr, nullptr, p->n_bins, 0,
+                               stream, 1, nullptr, 0, nullptr, &peak);
+}
+
 // Several plans of EQUAL geometry (one kernel bank per pitch: the note-relative transforms of a per-note iteration) in
 // as few launches as the 64-group argument block allows: plan i contracts clips [clip0[i], clip0[i] + nclips[i]) of the
 // batch whose cascade `lv` describes.  All launches use the same K split (the caller's finish kernel runs once).
 int cqt_stream_exec_multi(const saga_cqt_plan* const* plans, int n_plans, const int* clip0, const int* nclips,
                           const CqtLevels& lv, int n_clips, int64_t T_max, const int32_t* frame_first, int frame_count,
                           float* mag_out, float2* cplx_out, int64_t frame_pitch, int64_t out_clip_stride,
-                          cudaStream_t stream, int max_slices, float* partial, int pstride, int* slices_out) {
+                          cudaStream_t stream, int max_slices, float* partial, int pstride, int* slices_out,
+                          const CqtPeakArgs* peak) {
   if (n_plans < 1) return SAGA_OK;
   const saga_cqt_plan* p = plans[0];
   const CqtStreamState* st = p->stream_tc;
@@ -875,7 +950,7 @@ int cqt_stream_exec_multi(const saga_cqt_plan* const* plans, int n_plans, const 
       while (2 * ks <= max_slices && items * ks < n_sm && min_st / (2 * ks) >= 8 && min_st % (2 * ks) == 0) ks *= 2;
   }
   if (slices_out) *slices_out = ks;
-  if (frame_pitch > p->n_bins && ks == 1) {      // (the split-K finish kernel writes the padding itself)
+  if (frame_pitch > p->n_bins && ks == 1 && !peak) {      // (the split-K finish kernel writes the padding itself)
     dim3 grid(frame_first ? 1 : 8, n_clips), block(32, 8);
     cqt_stream_zero_cols_kernel<<<grid, block, 0, stream>>>(mag_out, cplx_out, lv.clip_frames, frame_first ? frame_count : 0,
                                                             p->n_bins, frame_pitch, out_clip_stride);
@@ -895,6 +970,12 @@ int cqt_stream_exec_multi(const saga_cqt_plan* const* plans, int n_plans, const 
   a.n_oct = (int)p->oct.size();
   a.pstride = pstride;
   a.partial = partial;
+  if (peak) {        // rows are packed on the device: the launch is sized for n_clips * T_max, the kernel runs what exists
+    a.row_start = peak->row_start;
+    a.col_lo = peak->col_lo;
+    a.col_hi = peak->col_hi;
+    a.peak_out = reinterpret_cast<unsigned int*>(peak->peak_out);
+  }
   uint32_t item0 = 0;
   int ng = 0;
   for (int pi = p0; pi < p1; ++pi) {
@@ -973,7 +1054,8 @@ int cqt_stream_exec_multi(const saga_cqt_plan* const* plans, int n_plans, const 
   }
   const int grid = (int)std::min<int64_t>(a.total_items, n_sm);
   if (a.debug & (16 | 128)) cudaMemsetAsync(st->d_prof, 0, sizeof(long long) * (2048 + 96 * 8), stream);
-  cqt_umma_stream_kernel<<<grid, US_THREADS, smem_bytes, stream>>>(a);
+  if (peak) cqt_umma_stream_kernel<true><<<grid, US_THREADS, smem_bytes, stream>>>(a);
+  else cqt_umma_stream_kernel<false><<<grid, US_THREADS, smem_bytes, stream>>>(a);
   SAGA_LAUNCH_CHECK();
   if (a.debug & 128) {
     // profiling aid only: timeline of CTA 0's first 96 stages (cycles relative to the first event)

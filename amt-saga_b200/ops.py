@@ -317,6 +317,32 @@ def cqt_batch(wav, plan, lens=None, want_complex=False, impl=0, fill=None):
     return out
 
 
+def cqt_peak_batch(wav, plan, col_lo, col_hi, lens=None):
+    """saga_cqt_peak_exec: per clip, max |C| over every bin and the frames col_lo[c] <= t < min(col_hi[c], T_c)
+    (0 for an empty range) -- np.max of `C[:, lo:hi]` without the image.  col_lo / col_hi: int sequences or tensors
+    [clips].  Returns a float32 CUDA tensor [clips]."""
+    wav, offs, lens_dev, max_len = _clip_table(wav, lens)
+    n_clips = wav.shape[0]
+    lib = _lib.lib()
+    dev = wav.device
+
+    def cols(x, name):
+        t = torch.as_tensor(np.ascontiguousarray(x, dtype=np.int32), device=dev) \
+            if not isinstance(x, torch.Tensor) else x.to(device=dev, dtype=torch.int32).contiguous()
+        if t.shape != (n_clips,):
+            raise ValueError("%s must be [clips]" % name)
+        return t
+    lo, hi = cols(col_lo, "col_lo"), cols(col_hi, "col_hi")
+    peak = torch.empty((n_clips,), device=dev, dtype=torch.float32)
+    nbytes = lib.saga_cqt_peak_workspace_bytes(plan.handle, n_clips, max_len)
+    ws = _workspace(nbytes, dev)
+    with _on(wav, plan):
+        _lib.check(lib.saga_cqt_peak_exec(plan.handle, _ptr(wav), _ptr(offs), _ptr(lens_dev) if lens is not None else None,
+                                          n_clips, max_len, _ptr(lo), _ptr(hi), _ptr(peak), _ptr(ws), ws.numel(),
+                                          _stream(wav)), ParameterError)
+    return peak
+
+
 def cqt_frames_batch(wav, plan, frame_first, frame_count=8, lens=None, out=None):
     """saga_cqt_frames_exec: only columns [frame_first[c], frame_first[c] + frame_count) of each clip's CQT
     magnitude (what slice_C + _resize keep).  Returns compact frame-major storage [clips, frame_count, P]

@@ -273,6 +273,18 @@ int saga_cqt_frames_shared_multi_exec(const saga_cqt_plan* const* plans, int n_p
                                       int64_t frame_pitch, int64_t out_clip_stride, void* workspace,
                                       int64_t workspace_bytes, void* stream);
 
+/* Peak of a column range per clip, the whole-song normalisers of the producer loop (training.py:271-282: np.max of
+ * `C[:, 0:t]`): max |C[bin, t]| over all bins and frames col_lo[c] <= t < min(col_hi[c], T_c) of clip c, written to
+ * peak_out[c] (0 for an empty range).  col_lo / col_hi: device int32 [n_clips]; peak_out: device float [n_clips].
+ * Same cascade, margins and contraction arithmetic as saga_cqt_exec; no image is written for the plans the streamed
+ * tensor-core kernel runs (its rows are then the clips' frames packed back to back, not n_clips x T_max); the other
+ * plans contract into an image inside the workspace, which saga_cqt_peak_workspace_bytes covers. */
+int64_t saga_cqt_peak_workspace_bytes(const saga_cqt_plan* plan, int n_clips, int64_t max_len);
+int saga_cqt_peak_exec(const saga_cqt_plan* plan, const float* wav, const int64_t* clip_offsets,
+                       const int64_t* clip_lens, int n_clips, int64_t max_len,
+                       const int32_t* col_lo, const int32_t* col_hi, float* peak_out,
+                       void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------
  * K5  feature gather for the classifiers (training.py:333-388)
  * ---------------------------------------------------------------------- */
