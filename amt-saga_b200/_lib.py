@@ -66,6 +66,7 @@ SIGNATURES = {
     "saga_short_window_batch_exec": (_I, [_P, _P, _L, _L, _P, _I, _P, _I, _I, _I, _P, _F, _P, _P, _P, _L, _L, _I, _P]),
     "saga_gather_frames_exec": (_I, [_P, _P, _P, _P, _I, _I, _I, _L, _L, _L, _L, _P]),
     "saga_spectral_flatness_exec": (_I, [_P, _P, _I, _I, _I, _L, _L, _F, _P]),
+    "saga_window_slide_exec": (_I, [_P, _P, _I, _I, _I, _I, _L, _L, _P, _P, _P, _P, _I, _P, _P, _L, _P]),
 }
 
 _lib = None

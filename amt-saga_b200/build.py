@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsaga_b200.so")
-SOURCES = ["api.cu", "stft.cu", "stft_ring.cu", "istft_ring.cu", "subtract_db.cu", "cqt.cu", "cqt_umma.cu", "cqt_umma_stream.cu", "features.cu", "ingest.cu"]
+SOURCES = ["api.cu", "stft.cu", "stft_ring.cu", "istft_ring.cu", "subtract_db.cu", "cqt.cu", "cqt_umma.cu", "cqt_umma_stream.cu", "features.cu", "ingest.cu", "window_slide.cu"]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-shared", "-Xcompiler", "-fPIC", "-lcuda"]
 

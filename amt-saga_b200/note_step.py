@@ -46,15 +46,25 @@ class NoteStepBatch:
         self.stft = ops.get_stft_plan(self.N, self.hl, True, device=self.dev)
         self.nb = self.stft.n_bins
         self._fft_freq = np.linspace(0, float(sr) / 2, int(1 + self.N // 2), endpoint=True)   # util_audio.py:67
-        self.mag = self.ph = self.wav = None
-        self.fresh = True
-        self._dirty = None         # frames changed by the last subtract, while `wav` is an iSTFT of the previous magnitudes
-        self._wav_synced = False   # `wav` == iSTFT(magnitudes before the last subtract) (the original audio is not)
+        self.mag = self.ph = self.wav = self.wav_lens = None
+        self.state = None          # [W] int8: AUDIO / SYNCED / DIRTY / FULL (what `wav` holds, below)
+        self._dirty = None         # frames changed by the last subtract of the DIRTY windows
         self.incremental_istft = True   # False: every rebuild of `wav` inverts all T frames (A/B twin)
         self.share_cascade = True       # False: every pitch group runs its own decimation cascade; "per_plan": shared
                                         # cascade but one contraction launch per pitch (A/B twins)
         self._tone_fft = None
         self.full_cqt = False      # True: every slice_C transforms all 258 columns like the reference (A/B twin)
+
+    # What `wav[w, :wav_lens[w]]` holds -- the class's `_wf` and what the next step has to do to it:
+    AUDIO = 0    # real audio: not subtracted since `load` or since a slide of a window that had a waveform
+    SYNCED = 1   # the iSTFT of the current rows (rebuilt, no subtraction since)
+    DIRTY = 2    # the iSTFT of the rows before the last subtraction: the next step patches the frames it changed
+    FULL = 3     # stale (a subtraction of AUDIO rows, two subtractions, or a slide of a stale window): full iSTFT
+
+    @property
+    def _wav_synced(self):
+        """Some window's `wav` is an iSTFT the next subtraction can patch incrementally."""
+        return self.state is not None and bool(((self.state == self.SYNCED) | (self.state == self.DIRTY)).any())
 
     # ------------------------------------------------------------------ helpers (host, float64)
     def midi_tone_to_FFT(self, tone):          # util_audio.py:278-284
@@ -63,8 +73,26 @@ class NoteStepBatch:
 
     def _frames(self, seconds):
         """util_audio.py:264 for every window: floor(time * T * sr / len(wf)), float64, that order."""
-        x = np.asarray(seconds, dtype=np.float64) * self.T * self.sr / self.wav.shape[1]
+        x = np.asarray(seconds, dtype=np.float64) * self.T * self.sr / self.wav_lens
         return np.floor(x).astype(np.int64)
+
+    def _lens_arg(self, order=None):
+        """`lens` for the CQT entries: None when every window fills the buffer (the dense path)."""
+        if (self.wav_lens == self.wav.shape[1]).all():
+            return None
+        return self.wav_lens if order is None else self.wav_lens[order]
+
+    @staticmethod
+    def _length_ok(plan, lens):
+        """Per window: does librosa accept a signal of this length for `plan` (check_length, per distinct length)."""
+        u, inv = np.unique(np.asarray(lens, dtype=np.int64), return_inverse=True)
+        ok = np.ones(len(u), dtype=bool)
+        for i, n in enumerate(u):
+            try:
+                plan.check_length(int(n))
+            except ParameterError:
+                ok[i] = False
+        return ok[inv.reshape(-1)]
 
     _resize_tables = {}
 
@@ -102,54 +130,70 @@ class NoteStepBatch:
         return out
 
     # ------------------------------------------------------------------ state
-    def load(self, mag_storage, phase_storage, wav, song_ref_mag, ref_C, window_ref_mag=None):
+    def load(self, mag_storage, phase_storage, wav, song_ref_mag, ref_C, window_ref_mag=None, wav_lens=None):
         """Windows as `mid_wf.section(offset, None, timing_frames)` leaves them (training.py:284):
         mag_storage / phase_storage: frame-major [W, T, P] (columns of the SONG's STFT), wav [W, L] the matching
         waveform slices, song_ref_mag [W] = mid_wf.ref_mag (the features' normaliser, training.py:336),
         ref_C [W, 3] = (ref_C_1, ref_C_inst, ref_C_foc).  window_ref_mag: the `_ref_mag` the section carries -- None
         (default) when the song's had not been evaluated yet at `section` time, which is training.py's order: the
-        first subtraction then scales by the window's own maximum; pass the song's to model a stale copy."""
+        first subtraction then scales by the window's own maximum; pass the song's to model a stale copy.
+        wav_lens [W]: the length of each window's waveform (what the class's `len(wf)` is) when `wav` is a padded batch
+        of windows of different lengths; None = every window is wav.shape[1] samples."""
         f32 = lambda x: torch.as_tensor(np.asarray(x, dtype=np.float32) if not isinstance(x, torch.Tensor) else x,
                                         device=self.dev).to(torch.float32).contiguous()
         if mag_storage.shape[:2] != (self.W, self.T) or phase_storage.shape != mag_storage.shape:
             raise ValueError("expected [W, T, P] magnitude and phase storage")
         self.mag, self.ph = mag_storage.contiguous(), phase_storage.contiguous()
         self.wav = wav.to(device=self.dev, dtype=torch.float32).contiguous()
+        if wav_lens is None:
+            self.wav_lens = np.full(self.W, self.wav.shape[1], dtype=np.int64)
+        else:
+            self.wav_lens = np.asarray(wav_lens.cpu() if isinstance(wav_lens, torch.Tensor) else wav_lens,
+                                       dtype=np.int64).reshape(-1).copy()
+            if self.wav_lens.shape != (self.W,) or (self.wav_lens < 1).any() or (self.wav_lens > self.wav.shape[1]).any():
+                raise ValueError("wav_lens must be [W] with 1 <= len <= wav.shape[1]")
         self.song_ref = f32(song_ref_mag)
         self.inv_song_ref = 1.0 / self.song_ref
         rc = np.asarray(ref_C.cpu() if isinstance(ref_C, torch.Tensor) else ref_C, dtype=np.float64).reshape(self.W, 3)
         self.inv_ref_C = [f32(1.0 / rc[:, i]) for i in range(3)]
+        # the `ref_mag` the next subtraction of each window scales by (< 0: the window's maximum at that moment)
         if window_ref_mag is None:
-            _, self.stale_ref = ops.subtract_db_batch(self.mag, None, None, self.nb, want_D=False)   # max of each window
+            _, self._ref_init = ops.subtract_db_batch(self.mag, None, None, self.nb, want_D=False)   # max of each window
         else:
-            self.stale_ref = f32(window_ref_mag)   # `section` copied a cached ref_mag (util_audio.py:323)
-        self.fresh = True
-        self._dirty, self._wav_synced = None, False
+            self._ref_init = f32(window_ref_mag)   # `section` copied a cached ref_mag (util_audio.py:323)
+        self._ref_given = np.full(self.W, window_ref_mag is not None)
+        self.state = np.full(self.W, self.AUDIO, dtype=np.int8)
+        self._dirty = None
 
     # ------------------------------------------------------------------ one batched step
     def _cqt_prepare(self, L, lowest_midi, nbins, bpt, s, t, n_cols):
-        """Host side of one slice_C shape: the plan, the first column each window needs and the `_resize` map
-        relative to it (frame-window form) or absolute (full transform)."""
+        """Host side of one slice_C shape for windows of L[w] samples: the plan, which windows librosa accepts, the
+        first column each window needs and the `_resize` map relative to it (frame-window form) or absolute (full
+        transform)."""
         plan = ops.get_cqt_plan(self.sr, self.hl, midi_to_hz(lowest_midi), int(nbins), int(12 * bpt), 2, device=self.dev)
-        plan.check_length(int(L))
-        Tc = plan.num_frames(int(L))
+        L = np.broadcast_to(np.asarray(L, dtype=np.int64), np.shape(s))
+        ok = self._length_ok(plan, L)
+        u, inv = np.unique(L, return_inverse=True)
+        Tc = np.array([plan.num_frames(int(n)) for n in u], dtype=np.int64)[inv.reshape(-1)]
         src = self._resize_map(s, t, Tc, n_cols)                                     # C[:, s:t] -> _resize
         windowed = n_cols <= 8 and not self.full_cqt
         # whatever t - s is, `_resize` keeps columns of [s, s + n_cols): contract only those (K2 frame window)
-        first = np.clip(s, 0, max(Tc - 1, 0)).astype(np.int32)
+        first = np.clip(s, 0, np.maximum(Tc - 1, 0)).astype(np.int32)
         rel = np.where(src >= 0, src - first[:, None], -1).astype(np.int32) if windowed else src
         assert not windowed or rel.max(initial=-1) < n_cols
-        return plan, windowed, first, rel
+        return plan, windowed, first, rel, ok
 
-    def _cqt_run(self, wav, plan, windowed, first_dev, rel_dev, n_cols, nbins, inv_ref):
+    def _cqt_run(self, wav, plan, windowed, first_dev, rel_dev, n_cols, nbins, inv_ref, lens=None):
         if windowed:
-            C = ops.cqt_frames_batch(wav, plan, first_dev, n_cols)                   # [W', n_cols, Pc]
+            C = ops.cqt_frames_batch(wav, plan, first_dev, n_cols, lens=lens)        # [W', n_cols, Pc]
         else:
-            C = ops.cqt_batch(wav, plan)["mag_storage"]                              # [W', Tc, Pc]
+            C = ops.cqt_batch(wav, plan, lens=lens)["mag_storage"]                   # [W', Tc, Pc]
         return ops.gather_frames_batch(C, nbins, rel_dev, inv_ref)                   # / ref_C
 
     def _cqt_columns(self, wav, lowest_midi, nbins, bpt, s, t, n_cols, inv_ref):
-        plan, windowed, first, rel = self._cqt_prepare(wav.shape[1], lowest_midi, nbins, bpt, s, t, n_cols)
+        plan, windowed, first, rel, ok = self._cqt_prepare(wav.shape[1], lowest_midi, nbins, bpt, s, t, n_cols)
+        if not ok.all():
+            plan.check_length(int(wav.shape[1]))
         d = self._upload({"first": first, "rel": rel})
         return self._cqt_run(wav, plan, windowed, d["first"], d["rel"], n_cols, nbins, inv_ref)
 
@@ -162,12 +206,13 @@ class NoteStepBatch:
         onset = np.asarray(onset, dtype=np.float64).reshape(W)
         duration = np.asarray(duration, dtype=np.float64).reshape(W)
         pitch = np.asarray(pitch, dtype=np.int64).reshape(W)
-        if not self.fresh:
+        if (self.state >= self.DIRTY).any():
             # util_audio.py:88-106: wf is rebuilt from the subtracted magnitude and the original phase
             self._rebuild_wav()
         s, t = self._frames(onset), self._frames(onset + duration)
         out = {}
-        L = int(self.wav.shape[1])
+        Lw = self.wav_lens
+        lens = self._lens_arg()
         a0, c8 = note_to_midi("A0"), note_to_midi("C8")
         nf = self.instrument_frames
         # ---- host: every index table of the step, then ONE upload ------------------------------------------
@@ -179,20 +224,24 @@ class NoteStepBatch:
                         ("C_sw_inst", a0, (c8 - a0) * self.inst_bpt, self.inst_bpt, nf, 1),
                         ("C_sw_inst_foc_const", 60, self.instrument_bands, self.inst_bpt * 4, nf, 2))
         const_plans = {}
+        valid = np.ones(W, dtype=bool)
         for name, low, nbins, bpt, n_cols, _ in const_shapes:
-            plan, windowed, first, rel = self._cqt_prepare(L, low, nbins, bpt, s, t, n_cols)
-            const_plans[name] = (plan, windowed)
+            plan, windowed, first, rel, ok = self._cqt_prepare(Lw, low, nbins, bpt, s, t, n_cols)
+            const_plans[name] = (plan, windowed, ok)
+            valid &= ok
             host["first_" + name], host["rel_" + name] = first, rel
         # the two note-relative transforms have one kernel bank per pitch: windows are sorted by pitch once, every
         # pitch group contracts its <= 8 columns straight into its slice of ONE compact buffer, and one gather
         # (C[:, s:t] -> _resize -> / ref_C_foc) serves all windows
-        valid = np.ones(W, dtype=bool)
         order = np.argsort(pitch, kind="stable")
         host["order"], host["inv_order"] = order, np.argsort(order)
         s_s, t_s, p_s = s[order], t[order], pitch[order]
-        Tc = 1 + L // self.hl
+        L_s = Lw[order]
+        lens_s = self._lens_arg(order)
+        part = (lambda a, b: None) if lens_s is None else (lambda a, b: lens_s[a:b])
+        Tc = 1 + L_s // self.hl
         src_s = self._resize_map(s_s, t_s, Tc, nf)
-        first_s = np.clip(s_s, 0, max(Tc - 1, 0)).astype(np.int32)
+        first_s = np.clip(s_s, 0, np.maximum(Tc - 1, 0)).astype(np.int32)
         full = self.full_cqt
         host["first_s"] = first_s
         host["rel_s"] = src_s if full else np.where(src_s >= 0, src_s - first_s[:, None], -1)
@@ -214,27 +263,31 @@ class NoteStepBatch:
         out["F_sw_inst_foc"], out["F_sw_inst_foc_log10"], out["ph"] = fn["lin"], fn["log"], fn["phase"]
         # -- constant-Q inputs (training.py:340-346, :365-388); filter_scale 2 (util_audio.py:426)
         for name, low, nbins, bpt, n_cols, ref_i in const_shapes:
-            plan, windowed = const_plans[name]
+            plan, windowed, ok = const_plans[name]
             out[name] = self._cqt_run(self.wav, plan, windowed, d["first_" + name], d["rel_" + name], n_cols, nbins,
-                                      self.inv_ref_C[ref_i])
+                                      self.inv_ref_C[ref_i], lens=lens)
+            if not ok.all():        # librosa refuses these windows' lengths: the loop skips their files
+                out[name][torch.as_tensor(~ok, device=self.dev)] = float("nan")
         wav_s = self.wav.index_select(0, d["order"])
         inv_ref_s = self.inv_ref_C[2].index_select(0, d["order"])
         res = []
         for nbins, bpt, shift in ((self.instrument_bands, self.inst_bpt * 4, 0), (self.bins_velocity, 2, -10)):
             P = ops.frame_pitch(nbins)
-            buf = torch.zeros((W, Tc if full else nf, P), device=self.dev, dtype=torch.float32)
+            buf = torch.zeros((W, int(Tc.max()) if full else nf, P), device=self.dev, dtype=torch.float32)
             # pitch groups [a, b) of the sorted windows with their plans
-            groups, a = [], 0
+            groups, a, refused = [], 0, np.zeros(W, dtype=bool)
             while a < W:
                 b = a + int(np.searchsorted(p_s[a:], p_s[a], side="right"))
                 try:
                     plan = ops.get_cqt_plan(self.sr, self.hl, midi_to_hz(int(p_s[a]) + shift), int(nbins),
                                             int(12 * bpt), 2, device=self.dev)
-                    plan.check_length(L)
+                    ok = self._length_ok(plan, L_s[a:b])
+                    if not ok.any():
+                        plan.check_length(int(L_s[a]))
+                    refused[a:b] = ~ok
                     groups.append((a, b, plan))
                 except ParameterError:      # librosa: "Filter pass-band lies beyond Nyquist" -> the loop skips the file
-                    valid[order[a:b]] = False
-                    buf[a:b] = float("nan")
+                    refused[a:b] = True
                     groups.append((a, b, None))
                 a = b
             i = 0
@@ -244,7 +297,8 @@ class NoteStepBatch:
                     i += 1
                     continue
                 if full:
-                    buf[a:b] = ops.cqt_batch(wav_s[a:b], plan)["mag_storage"]
+                    C = ops.cqt_batch(wav_s[a:b], plan, lens=part(a, b))["mag_storage"]
+                    buf[a:b, :C.shape[1]] = C
                     i += 1
                     continue
                 # consecutive pitches of equal geometry (early factor, levels, kernel length) decimate the audio the same
@@ -254,10 +308,10 @@ class NoteStepBatch:
                         groups[j + 1][2].geometry() == plan.geometry():
                     j += 1
                 if j == i:
-                    ops.cqt_frames_batch(wav_s[a:b], plan, d["first_s"][a:b], nf, out=buf[a:b])
+                    ops.cqt_frames_batch(wav_s[a:b], plan, d["first_s"][a:b], nf, lens=part(a, b), out=buf[a:b])
                 else:
                     A, B = a, groups[j][1]
-                    token = ops.cqt_cascade_shared(wav_s[A:B], plan)
+                    token = ops.cqt_cascade_shared(wav_s[A:B], plan, lens=part(A, B))
                     run = groups[i:j + 1]
                     if self.share_cascade == "per_plan":      # one contraction launch per pitch (A/B twin)
                         for (ga, gb, gp) in run:
@@ -266,6 +320,9 @@ class NoteStepBatch:
                         ops.cqt_frames_from_cascade_multi(token, [g_[2] for g_ in run], [g_[0] - A for g_ in run],
                                                           [g_[1] - g_[0] for g_ in run], d["first_s"][A:B], nf, buf[A:B])
                 i = j + 1
+            if refused.any():
+                valid[order[refused]] = False
+                buf[torch.as_tensor(refused, device=self.dev)] = float("nan")
             g = ops.gather_frames_batch(buf, nbins, d["rel_s"], inv_ref_s)
             res.append(g.index_select(0, d["inv_order"]))
         foc, vel = res
@@ -281,19 +338,89 @@ class NoteStepBatch:
         magnitudes and a subtraction changes frames [o, o + tg) only: with n_fft = 4 hops a sample depends on 4
         frames, so the samples that change are [(o - 2) hop, (o + tg + 2) hop), computed from frames
         [o - 4, o + tg + 4): gather those rows, invert them (K4 on ~1/4 of the frames) and patch that sample range.
-        Same frames, same accumulation order per sample: the patched waveform equals the full rebuild."""
+        Same frames, same accumulation order per sample: the patched waveform equals the full rebuild.
+        Per window: FULL windows are inverted whole, DIRTY ones patched, AUDIO / SYNCED ones left alone -- at most one
+        K4 call of each kind for the batch.  The [W, L] buffer grows if hop * (T - 1) is wider than it."""
         d = self._dirty
-        m = self.N // (2 * self.hl)                      # frames on either side that reach a sample
-        if d is None or not self._wav_synced or not self.incremental_istft or d["F"] >= self.T:
+        full, dirty = self.state == self.FULL, self.state == self.DIRTY
+        if dirty.any() and (d is None or not self.incremental_istft or d["F"] >= self.T):
+            full, dirty = full | dirty, np.zeros_like(dirty)
+        Li = self.hl * (self.T - 1)
+        if full.all():
             self.wav = ops.istft_batch(self.stft, mag=self.mag, phase=self.ph, n_bins=self.nb)
-        elif d["any"]:
-            F, hop = d["F"], self.hl
-            y = ops.istft_batch(self.stft, mag=self.mag, phase=self.ph, n_bins=self.nb, frame0=d["fa32"], n_frames=F)   # [W, (F-1) hop]
-            idx = d["fa"][:, None] * hop + torch.arange(y.shape[1], device=self.dev)   # global sample of every sub sample
-            keep = (idx >= d["lo"][:, None]) & (idx < d["hi"][:, None])
-            self.wav.scatter_(1, idx, torch.where(keep, y, self.wav.gather(1, idx)))
+        else:
+            if self.wav.shape[1] < Li:
+                self.wav = torch.nn.functional.pad(self.wav, (0, Li - self.wav.shape[1]))
+            if dirty.any() and d["any"]:
+                F, hop = d["F"], self.hl
+                y = ops.istft_batch(self.stft, mag=self.mag, phase=self.ph, n_bins=self.nb, frame0=d["fa32"], n_frames=F)   # [W, (F-1) hop]
+                idx = d["fa"][:, None] * hop + torch.arange(y.shape[1], device=self.dev)   # global sample of every sub sample
+                keep = (idx >= d["lo"][:, None]) & (idx < d["hi"][:, None])
+                self.wav.scatter_(1, idx, torch.where(keep, y, self.wav.gather(1, idx)))
+            if full.any():
+                sel = torch.as_tensor(np.flatnonzero(full), device=self.dev)
+                y = ops.istft_batch(self.stft, mag=self.mag.index_select(0, sel), phase=self.ph.index_select(0, sel),
+                                    n_bins=self.nb)
+                self.wav.index_copy_(0, sel, torch.nn.functional.pad(y, (0, self.wav.shape[1] - y.shape[1])))
+        self.wav_lens[full | dirty] = Li
+        self.state[full | dirty] = self.SYNCED
         self._dirty = None
-        self._wav_synced = True
+
+    def wf(self):
+        """The class's `wf` getter for every window: pending rebuilds run now (the next step then has none) and
+        (wav [W, L], wav_lens [W] host) come back.  Like reading `audio_w.wf`, it leaves each window holding its
+        waveform, so a slide before the next subtraction cuts that waveform instead of dropping it."""
+        if (self.state >= self.DIRTY).any():
+            self._rebuild_wav()
+        return self.wav, self.wav_lens.copy()
+
+    def ref_mag(self):
+        """The class's `ref_mag` getter for every window (util_audio.py:170-174): the window's current maximum unless
+        one is cached, and caches it -- a slide keeps a cached value (slice / concat do not touch `_ref_mag`), so the
+        next subtraction scales by it instead of by the slid window's maximum.  Returns [W] float32 CUDA."""
+        need = ~self._ref_given
+        if need.any():
+            _, cur = ops.subtract_db_batch(self.mag, None, None, self.nb, want_D=False)   # max of each window now
+            self._ref_init = torch.where(torch.as_tensor(need, device=self.dev), cur, self._ref_init)
+            self._ref_given[:] = True
+        return self._ref_init
+
+    def _apply_slide(self, m, song_idx, g, song_mag, song_phase, song_wav):
+        """State side of a half-window slide (training.py:317-328) of windows m (host, distinct), with the host
+        geometry `song_setup.slide_geometry` gives: the rows (one slide-kernel launch), the waveforms and the
+        per-window state.  A window that holds a waveform (AUDIO / SYNCED) keeps `wf[a:b]` of it followed by the new
+        half's samples, one gather for all of them; any other window's `wf` is None in the class and becomes FULL: the
+        next step inverts all T rows."""
+        h = self.T // 2
+        m = np.asarray(m, dtype=np.int64)
+        ops.window_slide_batch(self.mag, self.ph, self.nb, h, m, song_idx, np.where(g["rows"] > 0, g["tfs"], 0), g["rows"],
+                               song_mag, song_phase)
+        has_wf = (self.state[m] == self.AUDIO) | (self.state[m] == self.SYNCED)
+        a, keep, n_copy, new_len = g["a"], g["keep"], g["n_copy"], g["wav_len"]
+        w0 = g["w0"]
+        ma = np.flatnonzero(has_wf)
+        cat = None
+        if len(ma):
+            Lc = int(new_len[ma].max())
+            d = self._upload({"row": m[ma], "a": a[ma], "keep": keep[ma], "song": np.asarray(song_idx)[ma],
+                              "w0": np.asarray(w0)[ma], "n_copy": np.asarray(n_copy)[ma]})
+            j = torch.arange(Lc, device=self.dev)[None, :]
+            kp, nc = d["keep"].long()[:, None], d["n_copy"].long()[:, None]
+            old = self.wav[d["row"].long()[:, None], (d["a"].long()[:, None] + j).clamp(max=self.wav.shape[1] - 1)]
+            new = song_wav[d["song"].long()[:, None], (d["w0"].long()[:, None] + j - kp).clamp(0, song_wav.shape[1] - 1)]
+            cat = torch.where(j < kp, old, torch.where((j >= kp) & (j < kp + nc), new, 0.0))
+        width = max(self.wav.shape[1], int(new_len.max()))
+        if width > self.wav.shape[1]:
+            self.wav = torch.nn.functional.pad(self.wav, (0, width - self.wav.shape[1]))
+        if cat is not None:
+            self.wav.index_copy_(0, d["row"].long(), torch.nn.functional.pad(cat, (0, width - cat.shape[1])))
+        self.wav_lens[m] = new_len
+        self.state[m] = np.where(has_wf, self.AUDIO, self.FULL).astype(np.int8)
+        # slice / concat keep `_ref_mag`: a copied one stays; None (subtracted, or never set) is the max at the next
+        # subtraction, which after the slide is the slid window's (util_audio.py:170-174)
+        drop = m[~self._ref_given[m]]
+        if len(drop):
+            self._ref_init = self._ref_init.index_fill(0, torch.as_tensor(drop, device=self.dev), -1.0)
 
     @staticmethod
     def _dirty_ranges(offset_frames, guess_frames, T, N, hop):
@@ -312,12 +439,15 @@ class NoteStepBatch:
         return F, fa, lo, hi, tg
 
     def _mark_dirty(self, offset_frames, guess_frames):
-        """Host side of the incremental rebuild: per window the frame range the subtraction touched."""
-        if not self._wav_synced or self._dirty is not None:
-            # `wav` is the original audio, or a second subtraction arrives before the rebuild: invert everything next time
-            self._dirty, self._wav_synced = None, False
+        """Host side of the incremental rebuild: per SYNCED window the frame range the subtraction touched.  Any other
+        window's `wav` is audio, or already stale (a second subtraction before the rebuild): it is inverted whole."""
+        syn = self.state == self.SYNCED
+        self.state = np.where(syn, self.DIRTY, self.FULL).astype(np.int8)
+        if not syn.any():
+            self._dirty = None
             return
-        F, fa, lo, hi, tg = self._dirty_ranges(offset_frames, guess_frames, self.T, self.N, self.hl)
+        tg_in = np.where(syn, np.asarray(guess_frames, dtype=np.int64), 0)
+        F, fa, lo, hi, tg = self._dirty_ranges(offset_frames, tg_in, self.T, self.N, self.hl)
         dev = self._upload({"fa": fa, "lo": lo, "hi": hi})
         self._dirty = {"F": F, "any": bool((tg > 0).any()), "fa32": dev["fa"], "fa": dev["fa"].long(), "lo": dev["lo"].long(),
                        "hi": dev["hi"].long()}
@@ -337,8 +467,9 @@ class NoteStepBatch:
         _, self.ref = ops.subtract_db_batch(
             self.mag, gm.unsqueeze(1),
             (offset_dev if offset_dev is not None else torch.as_tensor(offset_frames, dtype=torch.int32)).reshape(self.W, 1), self.nb,
-            guess_ref=g["clip_max"].reshape(self.W, 1), ref_init=self.stale_ref if self.fresh else self.ref,
+            guess_ref=g["clip_max"].reshape(self.W, 1), ref_init=self._ref_init,
             guess_frames=frames,
             normalize=True, relu=True, want_D=False)
-        self.stale_ref = None          # the `mag` setter dropped the copied ref_mag (util_audio.py:149-153)
-        self.fresh = False
+        # the `mag` setter dropped the copied ref_mag (util_audio.py:149-153); the next subtraction scales by the max
+        self._ref_init = self.ref
+        self._ref_given[:] = False

@@ -739,3 +739,50 @@ def spectral_flatness_batch(mag_storage, n_bins, amin=1e-10):
         _lib.check(_lib.lib().saga_spectral_flatness_exec(
             _ptr(m), _ptr(out), n_clips, n_bins, T, P, m.stride(0) if n_clips > 1 else T * P, float(amin), _stream(m)))
     return out
+
+
+def window_slide_batch(mag, phase, n_bins, half, windows, song_idx, song_row0, song_rows, song_mag, song_phase):
+    """saga_window_slide_exec: the producer loop's half-window slide (training.py:317-328), in place on the frame-major
+    window storages mag [W, T, P] float32 / phase [W, T, P] complex64 of the listed windows: rows [0, half) take rows
+    [half, 2 half), rows [half, 2 half) take rows [song_row0[i], song_row0[i] + half) of song song_idx[i] of
+    song_mag / song_phase [S, T_song, P] (zero from row song_rows[i] on).  windows / song_idx / song_row0 / song_rows:
+    int sequences or tensors [n] (one entry per listed window, windows distinct)."""
+    for t, name in ((mag, "mag"), (phase, "phase"), (song_mag, "song_mag"), (song_phase, "song_phase")):
+        _require_cuda(t, name)
+        if t.dim() != 3 or not t.is_contiguous():
+            raise ValueError("%s must be contiguous [clips, frames, P]" % name)
+    if mag.dtype != torch.float32 or song_mag.dtype != torch.float32 or phase.dtype != torch.complex64 \
+            or song_phase.dtype != torch.complex64:
+        raise ValueError("magnitudes are float32, phases complex64")
+    if phase.shape != mag.shape or song_phase.shape != song_mag.shape or song_mag.shape[2] != mag.shape[2]:
+        raise ValueError("phase / magnitude storages must match, with one frame pitch")
+    W, T, P = mag.shape
+    dev = mag.device
+
+    def ints(x, name):
+        t = torch.as_tensor(np.ascontiguousarray(x, dtype=np.int32), device=dev) \
+            if not isinstance(x, torch.Tensor) else x.to(device=dev, dtype=torch.int32).contiguous()
+        return t.reshape(-1)
+    if not isinstance(windows, torch.Tensor):       # host lists are checked here; device lists are the caller's
+        w_h = np.asarray(windows, dtype=np.int64).reshape(-1)
+        r0_h = np.asarray(song_row0, dtype=np.int64).reshape(-1)
+        nr_h = np.asarray(song_rows, dtype=np.int64).reshape(-1)
+        s_h = np.asarray(song_idx, dtype=np.int64).reshape(-1)
+        if ((w_h < 0) | (w_h >= W)).any() or len(np.unique(w_h)) != len(w_h):
+            raise ValueError("windows must be distinct indices in [0, %d)" % W)
+        if ((s_h < 0) | (s_h >= song_mag.shape[0])).any():
+            raise ValueError("song index out of range")
+        if len(r0_h) == len(nr_h):
+            live = np.minimum(nr_h, half)
+            if ((live > 0) & ((r0_h < 0) | (r0_h + live > song_mag.shape[1]))).any():
+                raise ValueError("live song rows past the song storage")
+    win, sidx, row0, rows = (ints(x, n) for x, n in ((windows, "windows"), (song_idx, "song_idx"),
+                                                     (song_row0, "song_row0"), (song_rows, "song_rows")))
+    n = win.numel()
+    if not (sidx.numel() == row0.numel() == rows.numel() == n):
+        raise ValueError("windows, song_idx, song_row0 and song_rows must have one entry per listed window")
+    with _on(mag):
+        _lib.check(_lib.lib().saga_window_slide_exec(
+            _ptr(mag), _ptr(phase), W, T, int(half), int(n_bins), P, T * P, _ptr(win), _ptr(sidx), _ptr(row0),
+            _ptr(rows), n, _ptr(song_mag), _ptr(song_phase), song_mag.shape[1] * P, _stream(mag)))
+    return mag, phase

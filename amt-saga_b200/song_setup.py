@@ -4,6 +4,7 @@
     training.py:266       spectral flatness gate (songs above 0.3 are skipped)         K1 by-product + flatness kernel
     training.py:271-282   ref_C_1 / ref_C_inst / ref_C_foc = np.max(slice_C(0, dur, T))  K2 peak mode (no image)
     training.py:284       audio_w = mid_wf.section(offset, None, 258)                   row / sample gathers
+    training.py:317-328   half-window slide (section + slice + concat)                  slide kernel + one sample gather
     training.py:289       fft_bin_min_const = midi_tone_to_FFT(60)
     training.py:336       song ref_mag                                                  K1 by-product
 
@@ -64,18 +65,44 @@ def section_geometry(T, lens, offset_s, n_frames, sr):
     return dict(tfs=tfs, tfe=tfe, w0=w0, w1=w1, n_copy=n_copy, pad=pad, wav_len=n_copy + pad)
 
 
+def slide_geometry(T, wav_len, has_wf, T_song, song_len, offset_s, half_seconds, sr, hop):
+    """Host side of the loop's half-window slide (training.py:317-328) of windows with T rows, waveforms of wav_len
+    samples (has_wf: the class's `_wf` is not None) and offsets offset_s, in songs of T_song frames / song_len samples:
+        offset += half_seconds; new = section(offset + half_seconds, None, h); slice(h, 2h); concat(new)
+    Returns section_geometry's entries for the new half plus offset_s (the new offset), a / b (`slice`'s sample
+    range, util_audio.py:351-365, python slice clipping), keep (= b - a samples kept), rows (live song rows of the
+    new half), past_end (tfs > T_song: the class appends more than h columns) and wav_len (the window's new waveform
+    length: keep + n_copy + pad with a waveform, hop (T - 1) -- the next iSTFT -- without)."""
+    if T % 2:
+        raise ValueError("slice(h, 2h) + concat of an odd T = %d leaves T - 1 frames" % T)
+    h = T // 2
+    L = np.asarray(wav_len, dtype=np.int64)
+    T_song = np.asarray(T_song, dtype=np.int64)
+    off = np.asarray(offset_s, dtype=np.float64) + half_seconds
+    g = section_geometry(T_song, song_len, off + half_seconds, h, sr)
+    a = np.minimum((h / T / sr * L * sr).astype(np.int64), L)
+    b = np.minimum((2 * h / T / sr * L * sr).astype(np.int64), L)
+    keep = np.maximum(b - a, 0)
+    g.update(offset_s=off, a=a, b=b, keep=keep, rows=np.clip(T_song - g["tfs"], 0, h), past_end=g["tfs"] > T_song,
+             wav_len=np.where(has_wf, keep + g["n_copy"] + g["pad"], hop * (T - 1)))
+    return g
+
+
 # ---------------------------------------------------------------------------------- windows
 class SongWindows:
     """What `mid_wf.section(offset, None, n_frames)` leaves, for W windows of a SongBatch:
     mag / phase: frame-major storage [W, n_frames, P] (float32 / complex64), zero past the song's end;
-    wav [W, max(wav_len)] float32, zero after each window's `wav_len[w]` samples; song_idx, and the host geometry
-    of `section_geometry` (tfs, tfe, w0, w1, n_copy, pad, wav_len).  A window that starts past the song's end has
-    n_frames zero rows here; the class's copy has tfe - T columns there ((sic) util_audio.py:318-321)."""
+    wav [W, max(wav_len)] float32, zero after each window's `wav_len[w]` samples; song_idx, offset_s (float64 [W],
+    the window's offset in seconds, training.py's `offset`), and the host geometry of `section_geometry` (tfs, tfe,
+    w0, w1, n_copy, pad, wav_len).  A window that starts past the song's end has n_frames zero rows here; the
+    class's copy has tfe - T columns there ((sic) util_audio.py:318-321).  After `SongBatch.slide` the geometry
+    entries of a slid window describe the half it appended, and wav_len is the window's whole waveform."""
 
-    def __init__(self, mag, phase, wav, song_idx, geometry):
+    def __init__(self, mag, phase, wav, song_idx, geometry, offset_s):
         self.mag, self.phase, self.wav, self.song_idx = mag, phase, wav, song_idx
         self.geometry = geometry
         self.wav_len = geometry["wav_len"]
+        self.offset_s = np.array(offset_s, dtype=np.float64)
 
     def stacked_wav(self):
         """[W, L] waveforms for NoteStepBatch.load, which takes windows of one length only."""
@@ -202,12 +229,50 @@ class SongBatch:
         idx = torch.as_tensor(g["w0"], device=self.dev)[:, None] + torch.arange(Lw, device=self.dev)[None, :]
         take = torch.arange(Lw, device=self.dev)[None, :] < torch.as_tensor(g["n_copy"], device=self.dev)[:, None]
         wav = torch.where(take, self.wav[sel[:, None], idx.clamp(0, self.wav.shape[1] - 1)], 0.0)
-        return SongWindows(mag.contiguous(), phase.contiguous(), wav, song_idx, g)
+        return SongWindows(mag.contiguous(), phase.contiguous(), wav, song_idx, g, offset_s)
 
     def load_into(self, step, windows):
         """NoteStepBatch.load with each window's song normalisers: song_ref_mag and ref_C.  window_ref_mag stays None:
-        `section` (training.py:284) runs before the song's ref_mag is first evaluated (:336)."""
+        `section` (training.py:284) runs before the song's ref_mag is first evaluated (:336).  Windows may have
+        waveforms of different lengths (songs of different len / T ratios)."""
         idx = windows.song_idx
-        step.load(windows.mag, windows.phase, windows.stacked_wav(),
-                  self.ref_mag.index_select(0, torch.as_tensor(idx, device=self.dev)), self.ref_C[idx])
+        step.load(windows.mag, windows.phase, windows.wav,
+                  self.ref_mag.index_select(0, torch.as_tensor(idx, device=self.dev)), self.ref_C[idx],
+                  wav_lens=windows.wav_len)
         return step
+
+    def slide(self, step, windows, mask, half_seconds=3.0):
+        """training.py:317-328 for the windows where `mask` is set, on the state `load_into` gave `step`:
+            offset += half_seconds
+            new = mid_wf.section(offset + half_seconds, None, h)      # h = T // 2 rows of the song
+            audio_w.slice(h, 2h); audio_w.concat(new)
+        Rows: one slide-kernel launch for all masked windows.  Waveforms: a window that holds one (no subtraction since
+        it was loaded or last slid, or `step.wf()` was read since) keeps `wf[a:b]` plus the new half's samples, a
+        ragged length; any other window is inverted whole by the next step.  Updates windows.offset_s, the geometry and
+        wav_len of the slid windows.  Calling it twice before a step slides twice, as the loop does.
+        Returns a bool mask [W] of the windows whose new half starts past the song's end (tfs > T_song): the class
+        then appends tfe - T_song > h zero columns ((sic) util_audio.py:318-321), a window this batch cannot hold.
+        Their rows are zero-filled as `section` does, and from there on they differ from the class's."""
+        W, T = step.W, step.T
+        if T % 2:
+            raise ValueError("slice(h, 2h) + concat of an odd T = %d leaves T - 1 frames" % T)
+        if step.hl != self.hl or step.sr != self.sr:
+            raise ValueError("the step and the songs must share hop and sample rate")
+        mask = np.asarray(mask, dtype=bool).reshape(-1)
+        if mask.shape != (W,) or len(windows.song_idx) != W:
+            raise ValueError("mask must be [W], one entry per window of the batch")
+        past = np.zeros(W, dtype=bool)
+        m = np.flatnonzero(mask)
+        if not len(m):
+            return past
+        sidx = windows.song_idx[m]
+        has_wf = (step.state[m] == step.AUDIO) | (step.state[m] == step.SYNCED)
+        g = slide_geometry(T, step.wav_lens[m], has_wf, self.T[sidx], self.lens[sidx], windows.offset_s[m], half_seconds,
+                           self.sr, self.hl)
+        step._apply_slide(m, sidx, g, self.mag, self.phase, self.wav)
+        windows.offset_s[m] = g["offset_s"]
+        windows.wav_len = windows.geometry["wav_len"] = step.wav_lens.copy()
+        for k in ("tfs", "tfe", "w0", "w1", "n_copy", "pad"):
+            windows.geometry[k][m] = g[k]
+        past[m] = g["past_end"]
+        return past

@@ -322,6 +322,20 @@ int saga_gather_frames_exec(const float* in, const int32_t* src_frames, const fl
                             int n_windows, int n_cols, int n_bins, int64_t frame_pitch, int64_t clip_stride,
                             int64_t out_pitch, int64_t out_clip_stride, void* stream);
 
+/* Half-window slide of the producer loop (training.py:317-328: util_audio.py:351-365 `slice(h, 2h)` then :368-382
+ * `concat(section(offset + half, None, h))`) for the n_list windows windows[i] (device int32) of a batch of
+ * n_windows frame-major windows [n_windows][n_frames][frame_pitch] (mag float32, phase complex64 = float2), in place:
+ *   rows [0, half)       <- rows [half, 2 half)
+ *   rows [half, 2 half)  <- rows [song_row0[i], song_row0[i] + half) of song song_idx[i] of song_mag / song_phase
+ *                           (stride song_clip_stride, same frame_pitch); rows j >= song_rows[i] are written as 0
+ * Rows [2 half, n_frames) and windows not listed are not touched.  Padding columns: 16-byte chunks past n_bins are
+ * not touched, lanes of the last partial chunk are written as 0.  All storages 16-byte aligned, frame_pitch a
+ * multiple of 4.  One launch whatever n_list is. */
+int saga_window_slide_exec(float* mag, void* phase, int n_windows, int n_frames, int half, int n_bins,
+                           int64_t frame_pitch, int64_t clip_stride, const int32_t* windows, const int32_t* song_idx,
+                           const int32_t* song_row0, const int32_t* song_rows, int n_list, const float* song_mag,
+                           const void* song_phase, int64_t song_clip_stride, void* stream);
+
 /* util_audio.py:330-332 librosa.feature.spectral_flatness(power=2): flatness_out[clip*n_frames + t] */
 int saga_spectral_flatness_exec(const float* mag, float* flatness_out, int n_clips, int n_bins, int n_frames,
                                 int64_t frame_pitch, int64_t clip_stride, float amin, void* stream);
