@@ -53,6 +53,7 @@ class NoteStepBatch:
         self.share_cascade = True       # False: every pitch group runs its own decimation cascade; "per_plan": shared
                                         # cascade but one contraction launch per pitch (A/B twins)
         self._tone_fft = None
+        self._plan_frames = {}     # (note shape, distinct window lengths) -> [128 pitches, lengths] frame counts
         self.full_cqt = False      # True: every slice_C transforms all 258 columns like the reference (A/B twin)
 
     # What `wav[w, :wav_lens[w]]` holds -- the class's `_wf` and what the next step has to do to it:
@@ -197,6 +198,48 @@ class NoteStepBatch:
         d = self._upload({"first": first, "rel": rel})
         return self._cqt_run(wav, plan, windowed, d["first"], d["rel"], n_cols, nbins, inv_ref)
 
+    def _pitch_groups(self, p_s, L_s, nbins, bpt, shift):
+        """Runs [a, b) of equal pitch in the pitch-sorted windows with the plan of the note-relative shape (lowest note
+        pitch + shift); None where librosa refuses the plan.  Also the windows librosa refuses (plan or length)."""
+        W = len(p_s)
+        groups, a, refused = [], 0, np.zeros(W, dtype=bool)
+        while a < W:
+            b = a + int(np.searchsorted(p_s[a:], p_s[a], side="right"))
+            try:
+                plan = ops.get_cqt_plan(self.sr, self.hl, midi_to_hz(int(p_s[a]) + shift), int(nbins), int(12 * bpt), 2,
+                                        device=self.dev)
+                ok = self._length_ok(plan, L_s[a:b])
+                if not ok.any():
+                    plan.check_length(int(L_s[a]))
+                refused[a:b] = ~ok
+                groups.append((a, b, plan))
+            except ParameterError:      # librosa: "Filter pass-band lies beyond Nyquist" -> the loop skips the file
+                refused[a:b] = True
+                groups.append((a, b, None))
+            a = b
+        return groups, refused
+
+    def _note_frames(self, si, groups, starts, p_s, Tc0, u_len, inv_len):
+        """Frames of each (pitch-sorted) window's transform for note-relative shape si: the plan's count, which early
+        decimation can make 1 + L // hop + 1.  A table per shape and set of window lengths holds each pitch's counts,
+        so a step only computes the pitches it has not seen (0 = unknown; refused plans keep Tc0 = 1 + L // hop)."""
+        key = (si, u_len.tobytes())
+        tab = self._plan_frames.get(key)
+        if tab is None:
+            tab = self._plan_frames[key] = np.zeros((128, len(u_len)), dtype=np.int64)
+        if p_s[0] < 0 or p_s[-1] > 127:          # (sorted) pitches outside MIDI's range: no table, every group computed
+            Tc = Tc0.copy()
+            for a, b, plan in groups:
+                if plan is not None:
+                    Tc[a:b] = np.array([plan.num_frames(int(n)) for n in u_len], dtype=np.int64)[inv_len[a:b]]
+            return Tc
+        for g in np.flatnonzero(tab[p_s[starts], 0] == 0):
+            a, b, plan = groups[g]
+            if plan is not None:
+                tab[p_s[a]] = [plan.num_frames(int(n)) for n in u_len]
+        known = tab[p_s, inv_len]
+        return np.where(known > 0, known, Tc0)
+
     def step(self, onset, duration, pitch, guess_wav, guess_lens=None, subtract=True):
         """onset / duration (seconds, relative to the window) and MIDI pitch per window (host arrays, [W]);
         guess_wav [W, Lg]: the rendered guessed notes (device float32; `guess_lens` for ragged renders).
@@ -239,12 +282,14 @@ class NoteStepBatch:
         L_s = Lw[order]
         lens_s = self._lens_arg(order)
         part = (lambda a, b: None) if lens_s is None else (lambda a, b: lens_s[a:b])
-        Tc = 1 + L_s // self.hl
-        src_s = self._resize_map(s_s, t_s, Tc, nf)
-        first_s = np.clip(s_s, 0, np.maximum(Tc - 1, 0)).astype(np.int32)
         full = self.full_cqt
-        host["first_s"] = first_s
-        host["rel_s"] = src_s if full else np.where(src_s >= 0, src_s - first_s[:, None], -1)
+        # the `_resize` maps for 1 + L // hop frames; a note-relative plan with early decimation can have one frame more,
+        # and the windows whose slice reaches that frame get their own rows below
+        Tc0 = 1 + L_s // self.hl
+        src0 = self._resize_map(s_s, t_s, Tc0, nf)
+        first0 = np.clip(s_s, 0, np.maximum(Tc0 - 1, 0)).astype(np.int32)
+        host["first_s"] = first0
+        host["rel_s"] = src0 if full else np.where(src0 >= 0, src0 - first0[:, None], -1)
         off = np.maximum(s, 0).astype(np.int32)       # util_audio.py:248 with attack_compensation 0
         host["off"] = off
         d = self._upload(host)
@@ -271,25 +316,29 @@ class NoteStepBatch:
         wav_s = self.wav.index_select(0, d["order"])
         inv_ref_s = self.inv_ref_C[2].index_select(0, d["order"])
         res = []
-        for nbins, bpt, shift in ((self.instrument_bands, self.inst_bpt * 4, 0), (self.bins_velocity, 2, -10)):
+        if len(self._plan_frames) > 256:       # windows of ever new lengths (song walks): keep the cache bounded
+            self._plan_frames.clear()
+        if lens_s is None:
+            u_len, inv_len = L_s[:1], np.zeros(W, dtype=np.int64)
+        else:
+            u_len, inv_len = np.unique(L_s, return_inverse=True)
+            inv_len = inv_len.reshape(-1)
+        starts = np.flatnonzero(np.r_[True, p_s[1:] != p_s[:-1]])      # the pitch groups' first windows
+        note_shapes = ((self.instrument_bands, self.inst_bpt * 4, 0), (self.bins_velocity, 2, -10))
+        for si, (nbins, bpt, shift) in enumerate(note_shapes):
             P = ops.frame_pitch(nbins)
+            groups, refused = self._pitch_groups(p_s, L_s, nbins, bpt, shift)
+            Tc = self._note_frames(si, groups, starts, p_s, Tc0, u_len, inv_len)
+            first_dev, rel_dev = d["first_s"], d["rel_s"]
+            r = np.flatnonzero((Tc != Tc0) & (np.maximum(s_s, t_s) >= np.minimum(Tc, Tc0) - 1))
+            if len(r):
+                src = self._resize_map(s_s[r], t_s[r], Tc[r], nf)
+                first = np.clip(s_s[r], 0, np.maximum(Tc[r] - 1, 0))
+                u = self._upload({"r": r, "first": first, "rel": src if full else np.where(src >= 0, src - first[:, None], -1)})
+                rows = u["r"].long()
+                first_dev = first_dev.index_copy(0, rows, u["first"])
+                rel_dev = rel_dev.index_copy(0, rows, u["rel"])
             buf = torch.zeros((W, int(Tc.max()) if full else nf, P), device=self.dev, dtype=torch.float32)
-            # pitch groups [a, b) of the sorted windows with their plans
-            groups, a, refused = [], 0, np.zeros(W, dtype=bool)
-            while a < W:
-                b = a + int(np.searchsorted(p_s[a:], p_s[a], side="right"))
-                try:
-                    plan = ops.get_cqt_plan(self.sr, self.hl, midi_to_hz(int(p_s[a]) + shift), int(nbins),
-                                            int(12 * bpt), 2, device=self.dev)
-                    ok = self._length_ok(plan, L_s[a:b])
-                    if not ok.any():
-                        plan.check_length(int(L_s[a]))
-                    refused[a:b] = ~ok
-                    groups.append((a, b, plan))
-                except ParameterError:      # librosa: "Filter pass-band lies beyond Nyquist" -> the loop skips the file
-                    refused[a:b] = True
-                    groups.append((a, b, None))
-                a = b
             i = 0
             while i < len(groups):
                 a, b, plan = groups[i]
@@ -308,22 +357,22 @@ class NoteStepBatch:
                         groups[j + 1][2].geometry() == plan.geometry():
                     j += 1
                 if j == i:
-                    ops.cqt_frames_batch(wav_s[a:b], plan, d["first_s"][a:b], nf, lens=part(a, b), out=buf[a:b])
+                    ops.cqt_frames_batch(wav_s[a:b], plan, first_dev[a:b], nf, lens=part(a, b), out=buf[a:b])
                 else:
                     A, B = a, groups[j][1]
                     token = ops.cqt_cascade_shared(wav_s[A:B], plan, lens=part(A, B))
                     run = groups[i:j + 1]
                     if self.share_cascade == "per_plan":      # one contraction launch per pitch (A/B twin)
                         for (ga, gb, gp) in run:
-                            ops.cqt_frames_from_cascade(token, gp, ga - A, gb - ga, d["first_s"][ga:gb], nf, buf[ga:gb])
+                            ops.cqt_frames_from_cascade(token, gp, ga - A, gb - ga, first_dev[ga:gb], nf, buf[ga:gb])
                     else:                                     # all pitches of the run in ~one launch per 10 banks
                         ops.cqt_frames_from_cascade_multi(token, [g_[2] for g_ in run], [g_[0] - A for g_ in run],
-                                                          [g_[1] - g_[0] for g_ in run], d["first_s"][A:B], nf, buf[A:B])
+                                                          [g_[1] - g_[0] for g_ in run], first_dev[A:B], nf, buf[A:B])
                 i = j + 1
             if refused.any():
                 valid[order[refused]] = False
                 buf[torch.as_tensor(refused, device=self.dev)] = float("nan")
-            g = ops.gather_frames_batch(buf, nbins, d["rel_s"], inv_ref_s)
+            g = ops.gather_frames_batch(buf, nbins, rel_dev, inv_ref_s)
             res.append(g.index_select(0, d["inv_order"]))
         foc, vel = res
         out["C_sw_inst_foc"], out["C_velocity"] = foc, vel

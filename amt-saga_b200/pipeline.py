@@ -50,7 +50,8 @@ class WindowFeaturePipeline:
         d, f32 = self.dev, torch.float32
         W = n_windows
         self.mag = torch.empty((W, self.T_clip, self.P), device=d, dtype=f32)
-        self.D = torch.empty((W, self.T_clip, self.P), device=d, dtype=f32)
+        # zeros: the dB pass writes the window's T rows only, and rows [T, T_clip) must not hold stale device memory
+        self.D = torch.zeros((W, self.T_clip, self.P), device=d, dtype=f32)
         self.frame_max = torch.empty((W, self.T_clip), device=d, dtype=f32)
         self.clip_max = torch.empty((W,), device=d, dtype=f32)
         self.gmag = torch.empty((W, 1, self.Tg, self.P), device=d, dtype=f32)

@@ -10,37 +10,8 @@ import amt_saga_b200  # noqa: F401
 from amt_saga_b200.cqt_plan import CqtPlan, ParameterError, kaiser_fast_taps
 from oracle import cqt as ocqt
 from oracle import resample as ors
-from oracle.spectral import note_to_hz, reflect_index
-
-
-def fir_decimate(x, taps, factor):
-    S = len(taps) - 1
-    n_full, n_out = len(x) // factor, -(-len(x) // factor)
-    h = np.concatenate([taps[:0:-1], taps]).astype(np.float64)
-    xp = np.concatenate([np.zeros(S), x, np.zeros(S + factor)])
-    idx = factor * np.arange(n_full)[:, None] + np.arange(2 * S + 1)[None, :]
-    y = np.zeros(n_out)
-    y[:n_full] = xp[idx] @ h
-    return y
-
-
-def device_model(plan, y):
-    y = np.asarray(y, dtype=np.float64)
-    levels = {0: fir_decimate(y, plan.early_taps, plan.early_factor) if plan.early_factor > 1 else y}
-    for l in range(1, plan.max_level + 1):
-        levels[l] = fir_decimate(levels[l - 1], plan.half_taps, 2)
-    T = plan.num_frames(len(y))
-    C = np.zeros((plan.n_bins, T), dtype=np.complex128)
-    for o in plan.octaves:
-        sig = levels[o["level"]]
-        n = np.arange(o["n_fft"])
-        idx = reflect_index(np.arange(T)[:, None] * o["hop"] + n[None, :] - o["n_fft"] // 2, len(sig))
-        out = sig[idx] @ o["bank"].astype(np.float64)          # [T, 2*n_filt]
-        for f in range(o["n_filters"]):
-            b = o["first_bin"] + f
-            if 0 <= b < plan.n_bins:
-                C[b] = out[:, 2 * f] + 1j * out[:, 2 * f + 1]
-    return C
+from oracle.spectral import midi_to_hz, note_to_hz
+from tests.step_replay import device_model
 
 
 CASES = [
@@ -50,6 +21,11 @@ CASES = [
     (44100, 1024, "A0", 87, 12),     # ref_C_1 (training.py:271): n_bins not a multiple of bpo
     (44100, 1024, "A0", 174, 24),    # C_sw_pitch (training.py:340)
     (44100, 1024, "D3", 36, 24),     # C_velocity (training.py:382): early factor 16
+    # the per-note step's heavy shapes (note_step.py), the plans tests/step_replay.py replays it with
+    (44100, 1024, "A0", 348, 48),    # C_sw_inst (training.py:344)
+    (44100, 1024, "C4", 348, 192),   # C_sw_inst_foc_const (training.py:375)
+    (44100, 1024, 93, 348, 192),     # C_sw_inst_foc at A6: the 12-pitch geometry run 93..104, no early decimation
+    (44100, 1024, 11, 36, 24),       # C_velocity of A0 (pitch - 10): early factor 128
 ]
 
 
@@ -60,7 +36,7 @@ def test_folded_banks_reproduce_oracle_cqt(sr, hop, low, n_bins, bpo):
     t = np.arange(n)
     y = 0.4 * np.sin(2 * np.pi * 220.0 * t / sr) + 0.2 * np.sin(2 * np.pi * 1318.5 * t / sr) \
         + 0.05 * rng.standard_normal(n)
-    fmin = note_to_hz(low)
+    fmin = note_to_hz(low) if isinstance(low, str) else float(midi_to_hz(low))     # a note name or a MIDI number
     ref = ocqt.cqt(y, sr=sr, hop_length=hop, fmin=fmin, n_bins=n_bins, bins_per_octave=bpo,
                    filter_scale=2)
     plan = CqtPlan(sr, hop, fmin, n_bins, bpo, filter_scale=2, create_device_plan=False)
