@@ -46,6 +46,7 @@ SIGNATURES = {
     "saga_stft_plan_destroy": (_I, [_P]),
     "saga_stft_num_frames": (_L, [_P, _L]),
     "saga_stft_exec": (_I, [_P, _P, _P, _P, _I, _L, _P, _P, _P, _L, _L, _P, _P, _P]),
+    "saga_stft_rows_exec": (_I, [_P, _P, _P, _P, _I, _P, _I, _P, _I, _I, _P, _P, _L, _L, _P, _P]),
     "saga_istft_exec": (_I, [_P, _P, _P, _P, _I, _I, _L, _L, _P, _L, _P]),
     "saga_istft_rows_exec": (_I, [_P, _P, _P, _P, _I, _P, _I, _L, _L, _P, _L, _P]),
     "saga_subtract_db_exec": (_I, [_P, _P, _L, _P, _P, _L, _P, _I, _P, _P, _P, _P, _P, _L, _I, _P, _P,

@@ -124,7 +124,8 @@ __device__ __forceinline__ void split_pair(float2 zk, float2 zm, float2 w, float
 // coalesced rows of the frame-major output, per-frame and per-clip maxima.
 template <int M, int R0, int R1, int R2, bool EXTRA, bool GT, int LANES = 32>
 __device__ __forceinline__ void stft_frame_out(const float2* buf, const float2* twN, const StftArgs& a, int clip,
-                                               int64_t t, int lane, int group = 0, float* gmax = nullptr) {
+                                               int64_t t, int dst, int64_t drow, int lane, int group = 0,
+                                               float* gmax = nullptr) {
   static_assert(LANES == 32 || R2 > 1, "multi-warp frames use the generic position map");
   // smem positions of Z[lane + 32 i] and of its partner Z[M - lane - 32 i] (digit-reversed order):
   //   zpos is affine in i for a fixed lane, so both are base + i * step
@@ -135,7 +136,7 @@ __device__ __forceinline__ void stft_frame_out(const float2* buf, const float2* 
   const int zm2 = pidx(zpos<M, R0, R1, R2>(M - lane - 64));
   const int zk_step = zk1 - zk0, zm_step = zm2 - zm1;
   // ---- real-FFT split, |X|, outputs -----------------------------------
-    const int64_t row = (int64_t)clip * a.out_clip_stride + t * a.frame_pitch;
+    const int64_t row = (int64_t)dst * a.out_clip_stride + drow * a.frame_pitch;
   float* mag_up = a.mag_out + row + lane;           // bins lane + LANES i
   float* mag_dn = a.mag_out + row + (M - lane);     // bins M - lane - LANES i
   const float2* twp = twN + lane;
@@ -228,8 +229,8 @@ __device__ __forceinline__ void dif_pass_last_regs(const float2* buf, float2 (&v
 
 template <int M, int R, bool EXTRA, bool GT>
 __device__ __forceinline__ void stft_frame_out_regs(const float2 (&v)[R], const float2* twN, const StftArgs& a,
-                                                    int clip, int64_t t, int lane) {
-  const int64_t row = (int64_t)clip * a.out_clip_stride + t * a.frame_pitch;
+                                                    int clip, int64_t t, int dst, int64_t drow, int lane) {
+  const int64_t row = (int64_t)dst * a.out_clip_stride + drow * a.frame_pitch;
   float* mag_up = a.mag_out + row + lane;           // bins lane + 32 i
   float* mag_dn = a.mag_out + row + (M - lane);     // bins M - lane - 32 i
   const float2* twp = twN + lane;
@@ -297,8 +298,55 @@ __device__ __forceinline__ void stft_frame_out_regs(const float2 (&v)[R], const 
 // threads that share one frame of the forward transform
 __host__ __device__ constexpr int stft_lanes(int M) { return M <= 1024 ? 32 : (M == 2048 ? 64 : 128); }
 
-template <int M, int R0, int R1, int R2, int WARPS, bool EXTRA>
-__global__ void __launch_bounds__(WARPS * 32, 2) stft_kernel(const StftArgs a) {
+// Frame range of saga_stft_rows_exec, a kernel argument of its own: StftArgs is embedded in the ring kernel's
+// arguments, whose layout stays as it is.
+struct StftRows {
+  const int32_t* frame0;     // clip c computes frames frame0[c] + j, j in [0, n_frames)
+  const int32_t* dst_clip;   // output clip of clip c (NULL: c)
+  int n_frames, dst_row0;    // frame j is written as row dst_row0 + j
+};
+
+// The frames a CTA transforms: nF consecutive frames t0 .. of the clip, frame t0 + f written as row orow0 + f of
+// output clip dst.  Returns false when there are none.
+//   stft_exec (ROWS false): tile `tile` of the clip's T frames, rows = frames of clip `clip`.
+//   rows entry (ROWS true): frames frame0[clip] + j for the tile's j range, rows dst_row0 + j of output clip
+//   dst_clip[clip]; the tile's frames outside [0, T) are written here as zero rows (magnitude 0, phasor (0, 0),
+//   padding columns included) -- what a song's storage holds past its end.
+template <bool ROWS, int THREADS>
+__device__ __forceinline__ bool stft_tile(const StftArgs& a, const StftRows& r, int clip, int tile, int64_t T,
+                                          int64_t& t0, int& nF, int& dst, int64_t& orow0) {
+  if constexpr (!ROWS) {
+    t0 = (int64_t)tile * a.frames_per_cta;
+    if (t0 >= T) return false;
+    nF = (int)min((int64_t)a.frames_per_cta, T - t0);
+    dst = clip;
+    orow0 = t0;
+    return true;
+  } else {
+    const int j0 = tile * a.frames_per_cta;
+    const int nJ = min(a.frames_per_cta, r.n_frames - j0);
+    const int64_t ts = (int64_t)r.frame0[clip] + j0;
+    const int lo = (int)min(max(-ts, (int64_t)0), (int64_t)nJ);     // frames before the clip's start
+    const int hi = (int)max(min(T - ts, (int64_t)nJ), (int64_t)lo);  // first frame at or past its end
+    dst = r.dst_clip ? r.dst_clip[clip] : clip;
+    orow0 = (int64_t)r.dst_row0 + j0;
+    float* mag = a.mag_out + (int64_t)dst * a.out_clip_stride + orow0 * a.frame_pitch;
+    float2* ph = a.phase_out ? a.phase_out + (int64_t)dst * a.out_clip_stride + orow0 * a.frame_pitch : nullptr;
+    const int64_t z0 = (int64_t)lo * a.frame_pitch, z1 = (int64_t)hi * a.frame_pitch, zn = (int64_t)nJ * a.frame_pitch;
+    for (int64_t i = threadIdx.x; i < z0 + (zn - z1); i += THREADS) {
+      const int64_t k = i < z0 ? i : z1 + (i - z0);
+      mag[k] = 0.f;
+      if (ph) ph[k] = make_float2(0.f, 0.f);
+    }
+    t0 = ts + lo;
+    nF = hi - lo;
+    orow0 += lo;
+    return nF > 0;
+  }
+}
+
+template <int M, int R0, int R1, int R2, int WARPS, bool EXTRA, bool ROWS = false>
+__global__ void __launch_bounds__(WARPS * 32, 2) stft_kernel(const StftArgs a, const StftRows rows) {
   constexpr int N = 2 * M;
   constexpr int BUF = M + M / 32;
   extern __shared__ __align__(16) float smem[];
@@ -312,9 +360,9 @@ __global__ void __launch_bounds__(WARPS * 32, 2) stft_kernel(const StftArgs a) {
   if (len <= 0) T = 0;
   else if (a.center) T = 1 + len / a.hop;
   else T = len >= N ? 1 + (len - N) / a.hop : 0;
-  const int64_t t0 = (int64_t)tile * a.frames_per_cta;
-  if (t0 >= T) return;
-  const int nF = (int)min((int64_t)a.frames_per_cta, T - t0);
+  int64_t t0, orow0;
+  int nF, dst;
+  if (!stft_tile<ROWS, WARPS * 32>(a, rows, clip, tile, T, t0, nF, dst, orow0)) return;
   const float* x = a.wav + a.clip_offsets[clip];
 
   // ---- stage the sample span once per CTA ---------------------------------
@@ -351,11 +399,11 @@ __global__ void __launch_bounds__(WARPS * 32, 2) stft_kernel(const StftArgs a) {
       // last pass stays in registers; bins k / M-k are paired by warp shuffles
       float2 v[R1];
       dif_pass_last_regs<M, L1, R1>(buf, v, lane);
-      stft_frame_out_regs<M, R1, EXTRA, true>(v, a.twN, a, clip, t0 + f, lane);
+      stft_frame_out_regs<M, R1, EXTRA, true>(v, a.twN, a, clip, t0 + f, dst, orow0 + f, lane);
     } else {
       dif_pass<M, L1, R1, false, (R2 == 1), true, LANES>(buf, nullptr, nullptr, a.tw1, lane, group);
       if constexpr (R2 > 1) dif_pass<M, L2, R2, false, true, true, LANES>(buf, nullptr, nullptr, nullptr, lane, group);
-      stft_frame_out<M, R0, R1, R2, EXTRA, true, LANES>(buf, a.twN, a, clip, t0 + f, lane, group, gmax);
+      stft_frame_out<M, R0, R1, R2, EXTRA, true, LANES>(buf, a.twN, a, clip, t0 + f, dst, orow0 + f, lane, group, gmax);
     }
     group_sync<LANES>(group);
   }
@@ -380,8 +428,8 @@ __device__ __forceinline__ void eo_store(const StftArgs& a, int64_t row, int k, 
   }
 }
 
-template <int WARPS, bool EXTRA>
-__global__ void __launch_bounds__(WARPS * 32, 2) stft_eo4096_kernel(const StftArgs a) {
+template <int WARPS, bool EXTRA, bool ROWS = false>
+__global__ void __launch_bounds__(WARPS * 32, 2) stft_eo4096_kernel(const StftArgs a, const StftRows rows) {
   constexpr int M = 2048, N = 4096, MH = 1024, BUFH = MH + MH / 32, GROUPS = WARPS / 2;
   extern __shared__ __align__(16) float smem[];
   __shared__ float gmax[WARPS];
@@ -395,9 +443,9 @@ __global__ void __launch_bounds__(WARPS * 32, 2) stft_eo4096_kernel(const StftAr
   if (len <= 0) T = 0;
   else if (a.center) T = 1 + len / a.hop;
   else T = len >= N ? 1 + (len - N) / a.hop : 0;
-  const int64_t t0 = (int64_t)tile * a.frames_per_cta;
-  if (t0 >= T) return;
-  const int nF = (int)min((int64_t)a.frames_per_cta, T - t0);
+  int64_t t0, orow0;
+  int nF, dst;
+  if (!stft_tile<ROWS, WARPS * 32>(a, rows, clip, tile, T, t0, nF, dst, orow0)) return;
   const float* x = a.wav + a.clip_offsets[clip];
 
   const int64_t s0 = t0 * a.hop - (a.center ? N / 2 : 0);
@@ -460,7 +508,7 @@ __global__ void __launch_bounds__(WARPS * 32, 2) stft_eo4096_kernel(const StftAr
 
     // ---- combine the halves + real-FFT split, 64 lanes: k = lane64 + 64 i in [0, 512) --------------------
     const int64_t t = t0 + f;
-    const int64_t row = (int64_t)clip * a.out_clip_stride + t * a.frame_pitch;
+    const int64_t row = (int64_t)dst * a.out_clip_stride + (orow0 + f) * a.frame_pitch;
     float vmax = 0.f;
 #pragma unroll 2
     for (int i = 0; i < 8; ++i) {
@@ -518,29 +566,31 @@ __global__ void __launch_bounds__(WARPS * 32, 2) stft_eo4096_kernel(const StftAr
   }
 }
 
-template <int WARPS>
-static int launch_stft_eo4096(const saga_stft_plan* p, const StftArgs& a, int n_clips, cudaStream_t st) {
+template <int WARPS, bool ROWS = false>
+static int launch_stft_eo4096(const saga_stft_plan* p, const StftArgs& a, int n_clips, cudaStream_t st,
+                              const StftRows& rows = StftRows{}) {
   const bool extra = a.phase_out || a.cplx_out;
-  auto kern = extra ? stft_eo4096_kernel<WARPS, true> : stft_eo4096_kernel<WARPS, false>;
+  auto kern = extra ? stft_eo4096_kernel<WARPS, true, ROWS> : stft_eo4096_kernel<WARPS, false, ROWS>;
   SAGA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   const int64_t blocks = (int64_t)n_clips * a.tiles_per_clip;
   if (blocks <= 0) return SAGA_OK;
   if (blocks > 0x7fffffffLL) return set_error(SAGA_ERR_INVALID, "stft: grid too large");
   if (a.frames_per_cta > WARPS / 2) return set_error(SAGA_ERR_INVALID, "stft: more frames per CTA than frame slots");
-  kern<<<(unsigned)blocks, WARPS * 32, p->smem_bytes, st>>>(a);
+  kern<<<(unsigned)blocks, WARPS * 32, p->smem_bytes, st>>>(a, rows);
   SAGA_LAUNCH_CHECK();
   return SAGA_OK;
 }
 
-template <int M, int R0, int R1, int R2, int WARPS>
-static int launch_stft(const saga_stft_plan* p, const StftArgs& a, int n_clips, cudaStream_t st) {
+template <int M, int R0, int R1, int R2, int WARPS, bool ROWS = false>
+static int launch_stft(const saga_stft_plan* p, const StftArgs& a, int n_clips, cudaStream_t st,
+                       const StftRows& rows = StftRows{}) {
   const bool extra = a.phase_out || a.cplx_out;
-  auto kern = extra ? stft_kernel<M, R0, R1, R2, WARPS, true> : stft_kernel<M, R0, R1, R2, WARPS, false>;
+  auto kern = extra ? stft_kernel<M, R0, R1, R2, WARPS, true, ROWS> : stft_kernel<M, R0, R1, R2, WARPS, false, ROWS>;
   SAGA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   const int64_t blocks = (int64_t)n_clips * a.tiles_per_clip;
   if (blocks <= 0) return SAGA_OK;
   if (blocks > 0x7fffffffLL) return set_error(SAGA_ERR_INVALID, "stft: grid too large");
-  kern<<<(unsigned)blocks, WARPS * 32, p->smem_bytes, st>>>(a);
+  kern<<<(unsigned)blocks, WARPS * 32, p->smem_bytes, st>>>(a, rows);
   SAGA_LAUNCH_CHECK();
   return SAGA_OK;
 }
@@ -933,6 +983,64 @@ extern "C" int saga_stft_exec(const saga_stft_plan* p, const float* wav, const i
     case 4096: return launch_stft<4096, 16, 16, 16, 8>(p, a, n_clips, st);
   }
   return set_error(SAGA_ERR_UNSUPPORTED, "stft_exec: unsupported n_fft");
+}
+
+extern "C" int saga_stft_rows_exec(const saga_stft_plan* p, const float* wav, const int64_t* clip_offsets,
+                                   const int64_t* clip_lens, int n_clips, const int32_t* frame0, int n_frames,
+                                   const int32_t* dst_clip, int dst_row0, int out_n_frames, float* mag_out,
+                                   void* phase_out, int64_t frame_pitch, int64_t out_clip_stride, float* clip_max_out,
+                                   void* stream) {
+  if (!p || !wav || !clip_offsets || !clip_lens || !frame0 || !mag_out)
+    return set_error(SAGA_ERR_INVALID, "stft_rows_exec: null argument");
+  if (n_clips < 0) return set_error(SAGA_ERR_INVALID, "stft_rows_exec: n_clips < 0");
+  if (n_frames <= 0) return set_error(SAGA_ERR_INVALID, "stft_rows_exec: n_frames %d <= 0", n_frames);
+  if (frame_pitch < p->M + 1)
+    return set_error(SAGA_ERR_INVALID, "stft_rows_exec: frame_pitch %lld < n_bins %d", (long long)frame_pitch, p->M + 1);
+  if (dst_row0 < 0 || (int64_t)dst_row0 + n_frames > out_n_frames)
+    return set_error(SAGA_ERR_INVALID, "stft_rows_exec: dst_row0 %d + n_frames %d outside the %d output rows", dst_row0,
+                     n_frames, out_n_frames);
+  if (out_clip_stride < (int64_t)out_n_frames * frame_pitch)
+    return set_error(SAGA_ERR_INVALID, "stft_rows_exec: out_clip_stride %lld < out_n_frames * frame_pitch",
+                     (long long)out_clip_stride);
+  if (n_clips == 0) return SAGA_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+
+  StftArgs a;
+  a.wav = wav;
+  a.clip_offsets = clip_offsets;
+  a.clip_lens = clip_lens;
+  a.mag_out = mag_out;
+  a.phase_out = (float2*)phase_out;
+  a.cplx_out = nullptr;
+  a.frame_max_out = nullptr;
+  a.clip_max_out = clip_max_out;
+  a.window = p->d_window_half;
+  a.tw0 = p->d_tw[0];
+  a.tw1 = p->d_tw[1];
+  a.twN = p->d_twN;
+  a.tw_eo = p->d_tw_eo;
+  a.frame_pitch = frame_pitch;
+  a.out_clip_stride = out_clip_stride;
+  a.hop = p->hop;
+  a.center = p->center;
+  a.frames_per_cta = p->frames_per_cta;
+  a.span_alloc = p->span_alloc;
+  a.tiles_per_clip = (n_frames + p->frames_per_cta - 1) / p->frames_per_cta;
+  a.max_frames = 0;
+  const StftRows r{frame0, dst_clip, n_frames, dst_row0};
+  // saga_stft_exec's kernel choice, so that a row equals that entry's row bit for bit -- except n_fft 2048 / hop 512,
+  // whose ring kernel stft_exec takes by default: the generic kernel here (stft_exec's SAGA_STFT_RING=0 twin)
+  switch (p->M) {
+    case 128: return launch_stft<128, 16, 8, 1, 8, true>(p, a, n_clips, st, r);
+    case 256: return launch_stft<256, 16, 16, 1, 8, true>(p, a, n_clips, st, r);
+    case 512: return launch_stft<512, 32, 16, 1, 8, true>(p, a, n_clips, st, r);
+    case 1024: return launch_stft<1024, 32, 32, 1, 10, true>(p, a, n_clips, st, r);
+    case 2048:
+      if (SAGA_OPT("SAGA_STFT_NO_EO")) return launch_stft<2048, 16, 16, 8, 8, true>(p, a, n_clips, st, r);
+      return launch_stft_eo4096<8, true>(p, a, n_clips, st, r);
+    case 4096: return launch_stft<4096, 16, 16, 16, 8, true>(p, a, n_clips, st, r);
+  }
+  return set_error(SAGA_ERR_UNSUPPORTED, "stft_rows_exec: unsupported n_fft");
 }
 
 static int istft_exec_impl(const saga_stft_plan* p, const void* cplx_in, const float* mag_in,

@@ -434,16 +434,25 @@ class NoteStepBatch:
             self._ref_given[:] = True
         return self._ref_init
 
-    def _apply_slide(self, m, song_idx, g, song_mag, song_phase, song_wav):
+    def _apply_slide(self, m, song_idx, g, song_mag, song_phase, song_wav, song_lens=None):
         """State side of a half-window slide (training.py:317-328) of windows m (host, distinct), with the host
         geometry `song_setup.slide_geometry` gives: the rows (one slide-kernel launch), the waveforms and the
         per-window state.  A window that holds a waveform (AUDIO / SYNCED) keeps `wf[a:b]` of it followed by the new
         half's samples, one gather for all of them; any other window's `wf` is None in the class and becomes FULL: the
-        next step inverts all T rows."""
+        next step inverts all T rows.  song_mag None: the songs are held as waveforms (song_wav [S, L], song_lens [S])
+        and the new halves' rows are computed from them."""
         h = self.T // 2
         m = np.asarray(m, dtype=np.int64)
-        ops.window_slide_batch(self.mag, self.ph, self.nb, h, m, song_idx, np.where(g["rows"] > 0, g["tfs"], 0), g["rows"],
-                               song_mag, song_phase)
+        if song_mag is None:
+            # with no live song rows the kernel only moves rows [h, 2h) down (and zeroes them): it never reads song
+            # storage, so the window storages stand in for it; the new halves then go straight into rows [h, 2h)
+            none = np.zeros(len(m), dtype=np.int64)
+            ops.window_slide_batch(self.mag, self.ph, self.nb, h, m, none, none, none, self.mag, self.ph)
+            ops.stft_rows_batch(song_wav, self.stft, g["tfs"], h, lens=song_lens, clip_rows=song_idx, out=self.mag,
+                                phase_out=self.ph, dst_clip=m, dst_row0=h)
+        else:
+            ops.window_slide_batch(self.mag, self.ph, self.nb, h, m, song_idx, np.where(g["rows"] > 0, g["tfs"], 0),
+                                   g["rows"], song_mag, song_phase)
         has_wf = (self.state[m] == self.AUDIO) | (self.state[m] == self.SYNCED)
         a, keep, n_copy, new_len = g["a"], g["keep"], g["n_copy"], g["wav_len"]
         w0 = g["w0"]
@@ -470,6 +479,33 @@ class NoteStepBatch:
         drop = m[~self._ref_given[m]]
         if len(drop):
             self._ref_init = self._ref_init.index_fill(0, torch.as_tensor(drop, device=self.dev), -1.0)
+
+    def _apply_refill(self, slots, wav, wav_lens, song_ref_mag, ref_C):
+        """State side of SongBatch.refill: windows `slots` (host, distinct), whose rows the caller has written, now hold
+        a fresh section -- waveform wav [n, >= max(wav_lens)], song_ref_mag [n], ref_C [n, 3] -- in the state `load`
+        leaves (AUDIO, the window's own maximum at its first subtraction).  The other windows keep theirs, bit for bit.
+        A refilled window that was DIRTY must leave the pending patch: `_rebuild_wav` writes its sample range
+        [lo, hi) into every window, so that range is emptied (hi = lo) -- otherwise the old rows' samples would land
+        in the new song's audio."""
+        slots = np.asarray(slots, dtype=np.int64)
+        sl = torch.as_tensor(slots, device=self.dev)
+        wav = wav.to(device=self.dev, dtype=torch.float32)
+        width = max(self.wav.shape[1], wav.shape[1])
+        if width > self.wav.shape[1]:
+            self.wav = torch.nn.functional.pad(self.wav, (0, width - self.wav.shape[1]))
+        self.wav.index_copy_(0, sl, torch.nn.functional.pad(wav, (0, width - wav.shape[1])))
+        self.wav_lens[slots] = np.asarray(wav_lens, dtype=np.int64)
+        ref = song_ref_mag.to(device=self.dev, dtype=torch.float32)
+        self.song_ref = self.song_ref.index_copy(0, sl, ref)
+        self.inv_song_ref = self.inv_song_ref.index_copy(0, sl, 1.0 / ref)
+        rc = np.asarray(ref_C, dtype=np.float64).reshape(len(slots), 3)
+        self.inv_ref_C = [c.index_copy(0, sl, torch.as_tensor((1.0 / rc[:, i]).astype(np.float32), device=self.dev))
+                          for i, c in enumerate(self.inv_ref_C)]
+        self._ref_init = self._ref_init.index_fill(0, sl, -1.0)
+        self._ref_given[slots] = False
+        self.state[slots] = self.AUDIO
+        if self._dirty is not None:
+            self._dirty["hi"] = self._dirty["hi"].index_copy(0, sl, self._dirty["lo"].index_select(0, sl))
 
     @staticmethod
     def _dirty_ranges(offset_frames, guess_frames, T, N, hop):

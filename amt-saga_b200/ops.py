@@ -272,6 +272,70 @@ def istft_batch(plan, F=None, mag=None, phase=None, n_bins=None, frame0=None, n_
     return wav
 
 
+def _int32_dev(x, dev, n, name, hi=None):
+    """int32 device [n] from host ints (range-checked against [0, hi) here) or a tensor (the caller's to check)."""
+    if isinstance(x, torch.Tensor):
+        t = x.to(device=dev, dtype=torch.int32).reshape(-1).contiguous()
+    else:
+        h = np.asarray(x, dtype=np.int64).reshape(-1)
+        if h.size == 1 and n != 1:
+            h = np.broadcast_to(h, (n,))
+        if (h < 0).any() or (hi is not None and (h >= hi).any()):
+            raise ValueError("%s out of range" % name)
+        t = torch.as_tensor(np.ascontiguousarray(h, dtype=np.int32), device=dev)
+    if t.numel() != n:
+        raise ValueError("%s must have one entry per clip" % name)
+    return t
+
+
+def stft_rows_batch(wav, plan, frame0, n_frames, lens=None, out=None, dst_clip=None, dst_row0=0, phase_out=None,
+                    clip_max=None, clip_rows=None):
+    """saga_stft_rows_exec, the forward twin of istft_batch(frame0=...): clip c computes frames frame0[c] + j,
+    j in [0, n_frames), of its own centred STFT and writes them as rows dst_row0 + j of output clip dst_clip[c] (of clip
+    c without dst_clip).  A row inside the clip equals stft_batch's row bit for bit; rows at or past its end are zero
+    (magnitude 0, phasor (0, 0)).
+        wav [rows, samples] CUDA float32 with `lens` as in stft_batch; clip_rows (ints [n]): clip c reads wav row
+            clip_rows[c] (default: clip c is row c) -- windows of songs without copying the songs;
+        frame0 / dst_clip: ints or int32 tensors [n] (one int broadcasts);
+        out: frame-major float32 [clips_out, T_out, P] (default: a new [n, n_frames, P]);
+        phase_out: complex64 storage shaped like `out`, or True for a new one;
+        clip_max: float32 [n] that takes the maximum over each clip's live rows WITHOUT being zeroed first (calls over
+            successive frame ranges accumulate ref_mag), or True for a new zeroed one.
+    Returns {"mag_storage", "phase_storage" (or None), "clip_max" (or None)}."""
+    wav, offs, lens_dev, _ = _clip_table(wav, lens)
+    dev = wav.device
+    if clip_rows is not None:
+        n = clip_rows.numel() if isinstance(clip_rows, torch.Tensor) else np.size(clip_rows)
+        sel = _int32_dev(clip_rows, dev, n, "clip_rows", wav.shape[0]).long()
+        offs, lens_dev = offs.index_select(0, sel), lens_dev.index_select(0, sel)
+    n_clips = offs.numel()
+    n_frames = int(n_frames)
+    P = frame_pitch(plan.n_bins)
+    if out is None:
+        out = torch.empty((n_clips, max(n_frames, 0), P), device=dev, dtype=torch.float32)
+    _require_cuda(out, "out")
+    if out.dim() != 3 or out.dtype != torch.float32 or not out.is_contiguous():
+        raise ValueError("out must be contiguous float32 [clips, T, P]")
+    if phase_out is True:
+        phase_out = torch.empty(out.shape, device=dev, dtype=torch.complex64)
+    if phase_out is not None and (phase_out.shape != out.shape or phase_out.dtype != torch.complex64
+                                  or not phase_out.is_contiguous()):
+        raise ValueError("phase_out must be contiguous complex64 shaped like out")
+    if clip_max is True:
+        clip_max = torch.zeros((n_clips,), device=dev, dtype=torch.float32)
+    if clip_max is not None and (clip_max.shape != (n_clips,) or clip_max.dtype != torch.float32):
+        raise ValueError("clip_max must be float32 [clips]")
+    f0 = _int32_dev(frame0, dev, n_clips, "frame0")
+    dc = None if dst_clip is None else _int32_dev(dst_clip, dev, n_clips, "dst_clip", out.shape[0])
+    n_out, T_out, Po = out.shape
+    with _on(wav, plan):
+        _lib.check(_lib.lib().saga_stft_rows_exec(
+            plan.handle, _ptr(wav), _ptr(offs), _ptr(lens_dev), n_clips, _ptr(f0), n_frames, _ptr(dc), int(dst_row0),
+            T_out, _ptr(out), _ptr(None if phase_out is None else torch.view_as_real(phase_out)), Po, T_out * Po,
+            _ptr(clip_max), _stream(wav)))
+    return {"mag_storage": out, "phase_storage": phase_out, "clip_max": clip_max}
+
+
 # ---------------------------------------------------------------------------
 # K2
 # ---------------------------------------------------------------------------

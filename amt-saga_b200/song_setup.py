@@ -116,10 +116,23 @@ class SongWindows:
 class SongBatch:
     """training.py:265-284 for a batch of songs.  The hyper-parameters are NoteStepBatch's: n_fft, hop (N / 4), sr,
     pitch_frames (slice_C's `magnitude_only` argument at training.py:271-282, truthy there) and the bins per tone of
-    the three whole-song CQTs (87 x 1, 87 x 4 and 87 x 16 bins from A0, i.e. 12 / 48 / 192 bins per octave)."""
+    the three whole-song CQTs (87 x 1, 87 x 4 and 87 x 16 bins from A0, i.e. 12 / 48 / 192 bins per octave).
+
+    hold: what the batch keeps of each song between calls.
+      "stft"      the whole song STFT, mag / phase [S, T_max, P] (24 624 B per frame at n_fft 4096: 6x the float32
+                  waveform); `section`, `slide` and `refill` gather their rows from it.
+      "waveform"  the waveforms only (mag / phase are None); `section`, `slide` and `refill` compute the rows they need
+                  with a frame-range STFT of the song (ops.stft_rows_batch).  Every row, waveform and normaliser equals
+                  hold="stft"'s bit for bit.  For corpora whose STFT does not fit the device."""
+
+    HOLDS = ("stft", "waveform")
+    chunk_bytes = 1 << 28      # hold="waveform" setup: magnitude scratch per chunk of frames, samples per CQT call
 
     def __init__(self, sr=44100, n_fft=4096, hop_length=None, pitch_frames=8, bins_per_tone=(1, 4, 16),
-                 flatness_threshold=0.3, lowest_note="A0", highest_note="C8", device=None):
+                 flatness_threshold=0.3, lowest_note="A0", highest_note="C8", device=None, hold="stft"):
+        if hold not in self.HOLDS:
+            raise ValueError("hold must be one of %s, not %r" % (self.HOLDS, hold))
+        self.hold = hold
         self.sr, self.N = sr, int(n_fft)
         self.hl = int(hop_length) if hop_length is not None else self.N // 4
         if not pitch_frames:
@@ -162,19 +175,26 @@ class SongBatch:
         """Runs training.py:265-284 for every song.  Sets (host arrays unless noted):
         T [S] frames, song_dur [S] float64, flatness [S] float64, keep [S] (flatness <= threshold), valid [S],
         ref_mag [S] float32 CUDA (the song's ref_mag), ref_C [S, 3] float64 (NaN where not valid), ref_cols [S] (the
-        column range [0, ref_cols) of the whole-song CQT maxima), and the song STFT as frame-major storage mag /
-        phase [S, T_max, P] (zero past each song's end).  Returns self."""
+        column range [0, ref_cols) of the whole-song CQT maxima), and under hold="stft" the song STFT as frame-major
+        storage mag / phase [S, T_max, P] (zero past each song's end; None under hold="waveform").  Returns self."""
         wav, lens = self._wave_in(songs, lens)
         S = wav.shape[0]
         self.wav, self.lens = wav, lens
-        # -- song STFT (training.py:269) and ref_mag (:336): one ragged K1 call
-        r = ops.stft_batch(wav, self.stft, lens=lens, want_phase=True, want_max=True)
-        self.mag, self.phase, self.ref_mag = r["mag_storage"], r["phase_storage"], r["clip_max"]
         self.T = song_frames(lens, self.hl)
+        if self.hold == "stft":
+            # -- song STFT (training.py:269) and ref_mag (:336): one ragged K1 call
+            r = ops.stft_batch(wav, self.stft, lens=lens, want_phase=True, want_max=True)
+            self.mag, self.phase, self.ref_mag = r["mag_storage"], r["phase_storage"], r["clip_max"]
+            T_max = self.mag.shape[1]
+            if T_max > 0:
+                flat = ops.spectral_flatness_batch(self.mag, self.nb)
+        else:
+            self.mag = self.phase = None
+            T_max = int(self.T.max(initial=0))
+            self.ref_mag, flat = self._song_frames_walk(T_max)
         # -- flatness gate (:266): mean over each song's own frames (a zero frame past the end would count as 1)
-        T_max = self.mag.shape[1]
         if T_max > 0:
-            flat = ops.spectral_flatness_batch(self.mag, self.nb).double()
+            flat = flat.double()
             T_dev = torch.as_tensor(self.T, device=self.dev)
             mask = torch.arange(T_max, device=self.dev)[None, :] < T_dev[:, None]
             self.flatness = (torch.where(mask, flat, 0.0).sum(1) / T_dev).cpu().numpy()
@@ -196,10 +216,62 @@ class SongBatch:
         lens_c = np.where(self.valid, lens, 0)
         lo = np.zeros(S, dtype=np.int32)
         hi = np.where(self.valid, self.ref_cols, 0).astype(np.int32)
-        peaks = [ops.cqt_peak_batch(wav, plan, lo, hi, lens=lens_c) for plan in self.cqt_plans]
+        if self.hold == "stft":
+            peaks = [ops.cqt_peak_batch(wav, plan, lo, hi, lens=lens_c) for plan in self.cqt_plans]
+        else:
+            # groups of songs of about chunk_bytes of samples: the CQT workspace scales with the songs of a call and
+            # would otherwise match the waveforms in size.  A clip's peak does not depend on the other clips of its call.
+            g = max(1, self.chunk_bytes // (4 * wav.shape[1]))
+            peaks = [torch.cat([ops.cqt_peak_batch(wav[s:s + g], plan, lo[s:s + g], hi[s:s + g], lens=lens_c[s:s + g])
+                                for s in range(0, S, g)]) for plan in self.cqt_plans]
         self.ref_C = torch.stack(peaks, dim=1).double().cpu().numpy()
         self.ref_C[~self.valid] = np.nan
         return self
+
+    def _song_frames_walk(self, T_max):
+        """hold="waveform" setup: the song STFT in chunks of frames, magnitudes only, through one reused buffer.
+        Returns ref_mag [S] (the maximum accumulates over the chunks) and the per-frame flatness [S, T_max] float32.
+        Both are per-frame quantities, so they equal hold="stft"'s bit for bit; the masked mean then runs once over
+        the whole table, in hold="stft"'s summation order."""
+        S = self.wav.shape[0]
+        ref = torch.zeros(S, device=self.dev, dtype=torch.float32)
+        if T_max == 0:
+            return ref, None
+        P = ops.frame_pitch(self.nb)
+        ch = max(1, min(T_max, self.chunk_bytes // (4 * P * S)))
+        buf = torch.empty(S * ch * P, device=self.dev, dtype=torch.float32)
+        flat = torch.empty((S, T_max), device=self.dev, dtype=torch.float32)
+        for c0 in range(0, T_max, ch):
+            n = min(ch, T_max - c0)
+            m = buf[:S * n * P].view(S, n, P)
+            ops.stft_rows_batch(self.wav, self.stft, c0, n, lens=self.lens, out=m, clip_max=ref)
+            flat[:, c0:c0 + n] = ops.spectral_flatness_batch(m, self.nb)
+        return ref, flat
+
+    def _section_rows(self, song_idx, tfs, n_frames):
+        """Rows tfs .. tfs + n_frames - 1 of songs song_idx, zero past each song's end: [n, n_frames, P] mag / phase."""
+        if self.hold == "waveform":
+            r = ops.stft_rows_batch(self.wav, self.stft, tfs, n_frames, lens=self.lens, clip_rows=song_idx, phase_out=True)
+            return r["mag_storage"], r["phase_storage"]
+        T = self.T[song_idx]
+        T_max = self.mag.shape[1]
+        sel = torch.as_tensor(song_idx, device=self.dev)
+        # frame rows tfs .. tfs + n_frames - 1, zero where they are past the song's end
+        rows = torch.as_tensor(tfs, device=self.dev)[:, None] + torch.arange(int(n_frames), device=self.dev)[None, :]
+        live = rows < torch.as_tensor(T, device=self.dev)[:, None]
+        rows_c = rows.clamp(max=max(T_max - 1, 0))
+        mag = torch.where(live[..., None], self.mag[sel[:, None], rows_c], 0.0)
+        phase = torch.where(live[..., None], self.phase[sel[:, None], rows_c], torch.zeros((), dtype=self.phase.dtype,
+                                                                                           device=self.dev))
+        return mag.contiguous(), phase.contiguous()
+
+    def _section_wav(self, song_idx, g):
+        """Samples [w0, w0 + n_copy) of songs song_idx, then zeros up to wav_len: [n, max(wav_len)]."""
+        sel = torch.as_tensor(song_idx, device=self.dev)
+        Lw = max(int(g["wav_len"].max(initial=0)), 1)
+        idx = torch.as_tensor(g["w0"], device=self.dev)[:, None] + torch.arange(Lw, device=self.dev)[None, :]
+        take = torch.arange(Lw, device=self.dev)[None, :] < torch.as_tensor(g["n_copy"], device=self.dev)[:, None]
+        return torch.where(take, self.wav[sel[:, None], idx.clamp(0, self.wav.shape[1] - 1)], 0.0)
 
     def section(self, song_idx, offset_s, n_frames=258):
         """`mid_wf.section(offset, None, n_frames)` (training.py:284, util_audio.py:286-328) of song song_idx[w] at
@@ -215,21 +287,8 @@ class SongBatch:
         T, lens = self.T[song_idx], self.lens[song_idx]
         g = section_geometry(T, lens, offset_s, n_frames, self.sr)
         g["song_idx"] = song_idx
-        T_max, P = self.mag.shape[1], self.mag.shape[2]
-        sel = torch.as_tensor(song_idx, device=self.dev)
-        # frame rows tfs .. tfs + n_frames - 1, zero where they are past the song's end
-        rows = torch.as_tensor(g["tfs"], device=self.dev)[:, None] + torch.arange(int(n_frames), device=self.dev)[None, :]
-        live = rows < torch.as_tensor(T, device=self.dev)[:, None]
-        rows_c = rows.clamp(max=max(T_max - 1, 0))
-        mag = torch.where(live[..., None], self.mag[sel[:, None], rows_c], 0.0)
-        phase = torch.where(live[..., None], self.phase[sel[:, None], rows_c], torch.zeros((), dtype=self.phase.dtype,
-                                                                                           device=self.dev))
-        # samples [w0, w0 + n_copy) of the song, then zeros up to wav_len
-        Lw = max(int(g["wav_len"].max(initial=0)), 1)
-        idx = torch.as_tensor(g["w0"], device=self.dev)[:, None] + torch.arange(Lw, device=self.dev)[None, :]
-        take = torch.arange(Lw, device=self.dev)[None, :] < torch.as_tensor(g["n_copy"], device=self.dev)[:, None]
-        wav = torch.where(take, self.wav[sel[:, None], idx.clamp(0, self.wav.shape[1] - 1)], 0.0)
-        return SongWindows(mag.contiguous(), phase.contiguous(), wav, song_idx, g, offset_s)
+        mag, phase = self._section_rows(song_idx, g["tfs"], n_frames)
+        return SongWindows(mag, phase, self._section_wav(song_idx, g), song_idx, g, offset_s)
 
     def load_into(self, step, windows):
         """NoteStepBatch.load with each window's song normalisers: song_ref_mag and ref_C.  window_ref_mag stays None:
@@ -246,7 +305,8 @@ class SongBatch:
             offset += half_seconds
             new = mid_wf.section(offset + half_seconds, None, h)      # h = T // 2 rows of the song
             audio_w.slice(h, 2h); audio_w.concat(new)
-        Rows: one slide-kernel launch for all masked windows.  Waveforms: a window that holds one (no subtraction since
+        Rows: one slide-kernel launch for all masked windows (under hold="waveform" the kernel only moves the rows down,
+        and one frame-range STFT of the songs writes the new halves).  Waveforms: a window that holds one (no subtraction since
         it was loaded or last slid, or `step.wf()` was read since) keeps `wf[a:b]` plus the new half's samples, a
         ragged length; any other window is inverted whole by the next step.  Updates windows.offset_s, the geometry and
         wav_len of the slid windows.  Calling it twice before a step slides twice, as the loop does.
@@ -256,8 +316,7 @@ class SongBatch:
         W, T = step.W, step.T
         if T % 2:
             raise ValueError("slice(h, 2h) + concat of an odd T = %d leaves T - 1 frames" % T)
-        if step.hl != self.hl or step.sr != self.sr:
-            raise ValueError("the step and the songs must share hop and sample rate")
+        self._check_step(step)
         mask = np.asarray(mask, dtype=bool).reshape(-1)
         if mask.shape != (W,) or len(windows.song_idx) != W:
             raise ValueError("mask must be [W], one entry per window of the batch")
@@ -269,10 +328,61 @@ class SongBatch:
         has_wf = (step.state[m] == step.AUDIO) | (step.state[m] == step.SYNCED)
         g = slide_geometry(T, step.wav_lens[m], has_wf, self.T[sidx], self.lens[sidx], windows.offset_s[m], half_seconds,
                            self.sr, self.hl)
-        step._apply_slide(m, sidx, g, self.mag, self.phase, self.wav)
+        step._apply_slide(m, sidx, g, self.mag, self.phase, self.wav, song_lens=self.lens)
         windows.offset_s[m] = g["offset_s"]
         windows.wav_len = windows.geometry["wav_len"] = step.wav_lens.copy()
         for k in ("tfs", "tfe", "w0", "w1", "n_copy", "pad"):
             windows.geometry[k][m] = g[k]
         past[m] = g["past_end"]
         return past
+
+    def _check_step(self, step):
+        if step.hl != self.hl or step.sr != self.sr:
+            raise ValueError("the step and the songs must share hop and sample rate")
+        if self.hold == "waveform" and step.N != self.N:
+            raise ValueError("the step and the songs must share n_fft")
+
+    def refill(self, step, windows, slots, song_idx, offset_s=0.0):
+        """Slot slots[i] of the batch `load_into` gave `step` now holds `section(song_idx[i], offset_s[i], step.T)`:
+        exactly what `section` + `load_into` give a fresh batch -- rows, waveform, song normalisers, the window's own
+        maximum as the first subtraction's ref_mag, state AUDIO -- while every other slot is left as it was, bit for
+        bit.  For a walk over more songs than slots: a slot whose song's notes are done, or whose slide went past the
+        song's end, takes the next song.  Updates windows.song_idx, offset_s, the geometry and wav_len of those slots.
+        Rows: one frame-range STFT straight into step.mag / step.ph (hold="waveform"), or a gather from the song STFT
+        (hold="stft")."""
+        slots = np.asarray(slots, dtype=np.int64).reshape(-1)
+        song_idx = np.asarray(song_idx, dtype=np.int64).reshape(-1)
+        offset_s = np.broadcast_to(np.asarray(offset_s, dtype=np.float64), song_idx.shape).copy()
+        if slots.shape != song_idx.shape:
+            raise ValueError("one song per refilled slot")
+        if ((slots < 0) | (slots >= step.W)).any() or len(np.unique(slots)) != len(slots):
+            raise ValueError("slots must be distinct indices in [0, %d)" % step.W)
+        if ((song_idx < 0) | (song_idx >= len(self.lens))).any():
+            raise ValueError("song index out of range")
+        if not self.valid[song_idx].all():
+            raise ValueError("songs that are not valid (empty or refused by the CQT)")
+        if (offset_s < 0).any():
+            raise ValueError("offsets must be >= 0")
+        if len(windows.song_idx) != step.W:
+            raise ValueError("windows must be the batch's, one entry per slot")
+        self._check_step(step)
+        if not len(slots):
+            return
+        g = section_geometry(self.T[song_idx], self.lens[song_idx], offset_s, step.T, self.sr)
+        if self.hold == "waveform":
+            ops.stft_rows_batch(self.wav, self.stft, g["tfs"], step.T, lens=self.lens, clip_rows=song_idx, out=step.mag,
+                                phase_out=step.ph, dst_clip=slots)
+        else:
+            mag, phase = self._section_rows(song_idx, g["tfs"], step.T)
+            sl = torch.as_tensor(slots, device=self.dev)
+            step.mag.index_copy_(0, sl, mag)
+            step.ph.index_copy_(0, sl, phase)
+        step._apply_refill(slots, self._section_wav(song_idx, g), g["wav_len"],
+                           self.ref_mag.index_select(0, torch.as_tensor(song_idx, device=self.dev)), self.ref_C[song_idx])
+        windows.song_idx = windows.song_idx.copy()
+        windows.song_idx[slots] = song_idx
+        windows.geometry["song_idx"] = windows.song_idx
+        windows.offset_s[slots] = offset_s
+        for k in ("tfs", "tfe", "w0", "w1", "n_copy", "pad"):
+            windows.geometry[k][slots] = g[k]
+        windows.wav_len = windows.geometry["wav_len"] = step.wav_lens.copy()

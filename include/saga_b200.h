@@ -98,6 +98,23 @@ int saga_stft_exec(const saga_stft_plan* plan, const float* wav,
                    int64_t frame_pitch, int64_t out_clip_stride, float* frame_max_out,
                    float* clip_max_out, void* stream);
 
+/* The same for a FRAME RANGE per clip (the forward twin of saga_istft_rows_exec): clip c computes frames
+ * t = frame0[c] + j, j in [0, n_frames), of its own centred STFT (reflect padding at the clip's true edges only) and
+ * writes frame j as row dst_row0 + j of output clip dst_clip[c] (of clip c when dst_clip is NULL); output clip d is at
+ * mag_out + d*out_clip_stride, out_n_frames rows of frame_pitch.  frame0 (int32) and dst_clip (int32) are device
+ * arrays [n_clips]; frame0[c] >= 0.
+ *   live rows (0 <= t < saga_stft_num_frames(len_c)) equal row t of saga_stft_exec on the same clip bit for bit, in
+ *     magnitude and phasor (same kernels; n_fft 2048 / hop 512 uses the generic kernel, stft_exec's SAGA_STFT_RING=0);
+ *   rows at or past the clip's end are zero rows: magnitude 0, phasor (0, 0);
+ *   padding columns [n_bins, frame_pitch) are 0.
+ * clip_max_out (optional, [n_clips], indexed by source clip) takes the atomic max over the live rows and is NOT
+ * zeroed here -- unlike saga_stft_exec, which zeroes its own -- so calls over successive frame ranges accumulate a
+ * clip's ref_mag.  phase_out is optional.  No per-frame maxima, no complex output. */
+int saga_stft_rows_exec(const saga_stft_plan* plan, const float* wav, const int64_t* clip_offsets,
+                        const int64_t* clip_lens, int n_clips, const int32_t* frame0, int n_frames,
+                        const int32_t* dst_clip, int dst_row0, int out_n_frames, float* mag_out, void* phase_out,
+                        int64_t frame_pitch, int64_t out_clip_stride, float* clip_max_out, void* stream);
+
 /* ------------------------------------------------------------------------
  * K4  inverse STFT (overlap-add), replaces librosa.istft reached from
  *   util_audio.py:92-104 (wf rebuilt from mag*ph after a subtraction)
